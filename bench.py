@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - throughput of the DIYGym step path on B200(s): aggregate env-steps/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--envs E] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--envs E] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one DIYGym.step for every environment (add-on update -> 2 x 1/480 s physics sub-steps with 150 solver
 sweeps -> observe/reward/terminal), synthetic uniform random actions.  Default workload = BASELINE.json configs[1]:
@@ -17,6 +17,14 @@ Printed JSON line (rank 0):
   cpu_baseline  the CPU oracle (kind "port", this repo's fp64 restatement - pybullet is absent) on the host cores
 With --impl reference the oracle itself is the timed arm (all host threads, bounded sample).
 Under torchrun (--gpus N > 1) every rank owns its own N environments (no per-step collective, weak scaling).
+
+--dump-outputs DIR writes what the last timed step left in rank 0's device buffers, as float32 DIR/<name>.npy: `state`
+(the physics state rows), `obs`, `reward`, `term` (the zero-width ones of a config are skipped) and `camera<k>_rgb` /
+`camera<k>_depth` per camera.  In configs with terminals, the step ends with the masked reset of finished episodes, and
+`reset` is 1 for the environments it restarted.  The reset observes them again, so in their rows `state`, `obs`,
+`reward` and `term` are post-reset values; the images are rendered before the reset.  Above 64 MB in all, a fixed sample of environments (seeded, the same rows in every
+array) is written instead; `env_index.npy` (float64) lists the environments written.  Actions, seeds and the step
+sequence depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -166,7 +174,12 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-per-config', action='store_true', help='skip the short runs of the other BASELINE.json configs (default run, 1 GPU)')
     ap.add_argument('--preroll', type=int, default=300, help='untimed steps before the warm-up (contact counts stationarise)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the CUDA step path (--impl ours)')
 
     rank = int(os.environ.get('RANK', 0))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
@@ -193,13 +206,10 @@ def main():
         vals, base = [], None
         for _ in range(warmup and 1):
             cpu_oracle_rate(env.scene, lo, hi, seconds=1.0)
-        t0 = time.perf_counter()
-        per = min(8.0, 120.0 / max(args.steps, 1))
-        for _ in range(max(args.steps, 1)):
+        per = min(8.0, 120.0 / args.steps)   # --steps timed samples of about 120 s in all
+        for _ in range(args.steps):
             base = cpu_oracle_rate(env.scene, lo, hi, seconds=per)
             vals.append(base['value'])
-            if time.perf_counter() - t0 > 150:
-                break
         v = float(np.median(vals))
         base['value'] = v
         line = {'impl': 'reference', 'metric': METRIC, 'value': v, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': args.steps, 'warmup': warmup,
@@ -218,13 +228,13 @@ def main():
     dev = torch.device('cuda', local_rank)
     torch.cuda.set_device(dev)
     ctx = dict(rank=rank, local_rank=local_rank, world_size=world_size, dev=dev, warmup=warmup, steps=args.steps, preroll=args.preroll, team=args.team)
-    main_res = measure(args.config, n_envs, ctx, cpu_baseline=not args.no_cpu_baseline, api_leg=True)
-    # the other BASELINE.json configs, one GPU only (driver-run numbers instead of builder-run claims): same measurement, shorter
+    main_res = measure(args.config, n_envs, ctx, cpu_baseline=not args.no_cpu_baseline, api_leg=True, dump_dir=args.dump_outputs)
+    # the other BASELINE.json configs, one GPU only: the same measurement with the same number of timed steps, shorter pre-roll
     per_config = None
     if world_size == 1 and not args.no_per_config and args.config == 'r2d2_maze' and not args.envs:
         per_config = {}
         for name in ('ur_high_5', 'from_the_readme', 'drone_pilot', 'ur_high_5_randomised'):
-            r = measure(name, CONFIGS[name][1], dict(ctx, steps=min(args.steps, 20), preroll=min(args.preroll, 200)), cpu_baseline=False, api_leg=False)
+            r = measure(name, CONFIGS[name][1], dict(ctx, preroll=min(args.preroll, 200)), cpu_baseline=False, api_leg=False)
             per_config['%s@%d' % (name, CONFIGS[name][1])] = {k: r[k] for k in ('value', 'ms_per_step', 'kernel_ms', 'e2e', 'roofline', 'gpu_launches', 'split_schedule')}
     if rank != 0:
         if world_size > 1:
@@ -245,11 +255,11 @@ def main():
     return 0
 
 
-def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True):
+def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True, dump_dir=None):
     """One configuration on this rank's GPU: pre-roll, K timed steps (device-resident actions, CUDA events, L2 flushed before
     every timed step), the host-buffer leg through dg_step_host, optionally the same loop through DIYGym.step(action dict), the
     roofline of the step launch sequence and the CPU oracle beside it.  Every rank calls this with the same arguments (the
-    barriers and the max-over-ranks reduction are inside)."""
+    barriers and the max-over-ranks reduction are inside).  dump_dir: rank 0 writes the outputs of the last timed step there."""
     import numpy as np
     import torch
     from diy_gym_b200 import DIYGym
@@ -266,6 +276,7 @@ def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True):
     user_addons = [a for r in env.receptors.values() for a in r.addons.values() if getattr(a, 'op', None) is None and a.action_space is not None]
     cams = [a for r in env.receptors.values() for a in r.addons.values() if type(a).__name__ == 'Camera']
     has_term = w.n_term > 0
+    last = {}   # the last step's images (views of buffers the next render overwrites) and reset mask, for --dump-outputs
 
     def device_step(i, render=True):
         if pool is not None:
@@ -274,10 +285,11 @@ def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True):
             a.update(torch.rand((n_envs, ) + tuple(a.action_space.shape), device=dev, generator=g))
         w.step()
         if render:
-            for c in cams:
-                w.render(c.cam)
+            for k, c in enumerate(cams):
+                last['camera%d_rgb' % k], last['camera%d_depth' % k] = w.render(c.cam)
         if has_term:
-            w.reset(w.term.amax(dim=1))   # masked reset of finished episodes, no host sync
+            last['reset'] = w.term.amax(dim=1)
+            w.reset(last['reset'])   # masked reset of finished episodes, no host sync
 
     def barrier():
         if world_size > 1:
@@ -319,6 +331,8 @@ def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True):
     launches = w.launches - l0
     clocks = sampler.stop() if sampler else None
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))   # average duration of a step's launches inside the timed region
+    if dump_dir and rank == 0:   # before the legs below step the world further
+        dump_outputs(dump_dir, dict(state=w.state, obs=w.obs, reward=w.reward, term=w.term, **last), n_envs)
 
     # ---- end to end through the host-buffer C-ABI call ----------------------------------------------------------
     pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory().numpy()
@@ -494,6 +508,25 @@ def measure(config, n_envs, ctx, cpu_baseline=True, api_leg=True):
     res.update(roofline=roofline, cpu_baseline=cpu)
     env.close()
     return res
+
+
+DUMP_LIMIT = 64 * 1000 * 1000   # bytes
+
+
+def dump_outputs(out_dir, arrays, n_envs):
+    """Writes each [n_envs, ...] device tensor of `arrays` as float32 out_dir/<name>.npy, zero-width ones skipped.  Above
+    DUMP_LIMIT bytes in all, the same seeded sample of environment rows is taken from every array."""
+    import numpy as np
+    import torch
+    arrays = {k: v for k, v in arrays.items() if v.numel()}
+    row_bytes = sum(4 * v[0].numel() for v in arrays.values()) + 8   # + the env_index entry
+    keep = min(n_envs, (DUMP_LIMIT - 128 * (len(arrays) + 1)) // row_bytes)   # 128: the header of a .npy file
+    idx = np.arange(n_envs) if keep == n_envs else np.sort(np.random.default_rng(0).choice(n_envs, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'env_index.npy'), idx.astype(np.float64))
+    rows = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), v.index_select(0, rows).float().cpu().numpy())
 
 
 def oracle_flops(scene, lo, hi, seed=1234):

@@ -143,3 +143,32 @@ def strict_single_step_parity(env, n_envs, steps, seed=4321, presteps=3, action_
         rec['term'] = (w.term.cpu().numpy(), np.stack([x[2] for x in outs]))
         recs.append(rec)
     return recs
+
+
+def golden_mesh(rel):
+    """(vertices, lo, hi) of source mesh `rel` from tests/golden/mesh_vertices.npz (tools/make_mesh_golden.py): vertices of the
+    mesh that include its extreme ones along each axis, and its bounding box, in the mesh frame."""
+    import os
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'mesh_vertices.npz'))
+    k = os.path.splitext(os.path.basename(rel))[0]
+    return g['verts_' + k], g['lo_' + k], g['hi_' + k]
+
+
+def write_mesh(path, verts):
+    """Writes a vertex cloud as a binary STL (triangles of consecutive vertices, the last one repeated to fill the last
+    triangle) or as a COLLADA file with one position source, chosen by the extension."""
+    import struct
+    v = np.asarray(verts, np.float64)
+    if path.endswith('.dae'):
+        floats = ' '.join('%.17g' % x for x in v.reshape(-1))
+        with open(path, 'w') as f:
+            f.write('<?xml version="1.0"?>\n<COLLADA xmlns="http://www.collada.org/2005/11/COLLADASchema" version="1.4.1">'
+                    '<library_geometries><geometry id="g"><mesh><source id="g-positions"><float_array id="g-positions-array" '
+                    'count="%d">%s</float_array></source><vertices id="g-vertices"><input semantic="POSITION" source="#g-positions"/>'
+                    '</vertices></mesh></geometry></library_geometries></COLLADA>\n' % (v.size, floats))
+        return
+    v = np.concatenate([v, np.repeat(v[-1:], -len(v) % 3, axis=0)]).astype('<f4').reshape(-1, 9)
+    with open(path, 'wb') as f:
+        f.write(b'\0' * 80 + struct.pack('<I', len(v)))
+        for tri in v:
+            f.write(struct.pack('<3f', 0, 0, 0) + tri.tobytes() + struct.pack('<H', 0))

@@ -14,6 +14,7 @@ from diy_gym_b200.assets import resolve_model
 from diy_gym_b200.compiler import mesh as cmesh
 from diy_gym_b200.compiler.scene import SceneBuilder
 from diy_gym_b200.compiler.urdf import compile_urdf, inertia_from_rule
+from tests.helpers import golden_mesh, write_mesh
 
 DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'diy_gym_b200', 'data')
 
@@ -84,22 +85,25 @@ B3 = {'ur5/meshes/collision/base.stl': ((-0.0736, -0.110, -0.003), (0.0736, 0.07
 
 
 @pytest.mark.parametrize('rel', sorted(B3))
-def test_mesh_reader_and_proxy_fit_against_the_survey_table(rel):
+def test_mesh_reader_and_proxy_fit_against_the_survey_table(rel, tmp_path):
     """The compiler's mesh reader gives the bounding box SURVEY B.3 lists, and the fitted collision proxy (capsule / box: meshes
     are not collided as hulls yet, DESIGN.md section 7) stays inside that box inflated by 15 % and covers at least 60 % of its
-    longest extent."""
-    path = None
-    for base in (DATA, '/root/reference/diy_gym/data'):
-        if os.path.isfile(os.path.join(base, rel)):
-            path = os.path.join(base, rel)
-            break
-    if path is None:
-        pytest.skip('mesh %s is not available here (compiled blobs only)' % rel)
+    longest extent.  The mesh files are not shipped: the test writes the vertices of the mesh kept in tests/golden (its
+    extreme vertices along each axis among them, so the same bounding box) as a binary STL and reads that.  fit_proxy
+    depends on nothing but the bounding box, so it fits the same proxy as to the whole mesh: the one the descriptor holds."""
+    verts, box_lo, box_hi = golden_mesh(rel)
+    path = str(tmp_path / os.path.basename(rel))
+    write_mesh(path, verts)
     v = cmesh.load_vertices(path)
     assert np.allclose(v, _stl_vertices(path))                               # the reader against an independent STL parse
+    assert np.allclose(v[:len(verts)], verts, rtol=1e-6, atol=1e-7)          # float32 round trip
     lo, hi = np.array(B3[rel][0]), np.array(B3[rel][1])
     assert np.allclose(v.min(axis=0), lo, atol=2e-3) and np.allclose(v.max(axis=0), hi, atol=2e-3)
+    assert np.allclose(v.min(axis=0), box_lo, atol=1e-7) and np.allclose(v.max(axis=0), box_hi, atol=1e-7)
     fit = cmesh.fit_proxy(v)
+    model = 'ur5/ur5_robot.urdf' if rel.startswith('ur5/') else 'hector_quadrotor/quadrotor.urdf'
+    col = next(c for l in resolve_model(model)['links'] for c in l['collisions'] if c.get('mesh') == os.path.basename(rel))
+    assert fit['type'] == col['type'] and np.allclose(fit['dims'], col['dims'][:len(fit['dims'])], atol=1e-7)
     c, half = np.array(fit['center']), np.array(fit['half'])
     ext = hi - lo
     assert np.all(c - half >= lo - 0.15 * ext.max()) and np.all(c + half <= hi + 0.15 * ext.max())

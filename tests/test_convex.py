@@ -12,19 +12,32 @@ from diy_gym_b200.compiler import mesh as cmesh
 from diy_gym_b200.compiler.mathutil import quat_to_mat
 from diy_gym_b200.compiler.scene import SceneBuilder
 from oracle.oracle import OracleWorld
+from tests.helpers import golden_mesh, write_mesh
 
-REF_DATA = '/root/reference/diy_gym/data'
 TOUCHING = [2.165, 0.011, 0.699, -1.475, 1.915, 1.938, 0.915, 0.138, -0.472, -0.662, 2.294, -0.915]   # joint angles of the two UR5s of examples/ur_high_5
 
 
 @pytest.mark.parametrize('rel', ['ur5/meshes/collision/forearm.stl', 'hector_quadrotor/meshes/quadrotor_base.stl', 'jaco/meshes/hand_3finger.dae'])
-def test_reduced_hull_approximates_the_mesh_from_inside(rel):
-    path = os.path.join(REF_DATA, rel)
-    if not os.path.isfile(path):
-        pytest.skip('mesh sources are only present in the build container (the repo ships compiled descriptors)')
+def test_reduced_hull_approximates_the_mesh_from_inside(rel, tmp_path):
+    """The mesh files are not shipped.  The cloud reduced here is made of the mesh vertices kept in tests/golden, points
+    inside their hull, and a seeded shell of points up to 1 % of the extent outside its facets, so that the reduction has to
+    thin far more than 32 hull vertices as it does on a real mesh.  It goes through the reader of the mesh's format."""
+    from scipy.spatial import ConvexHull
+    verts, _, _ = golden_mesh(rel)
+    rng = np.random.default_rng(7)
+    hull = ConvexHull(verts)
+    f = rng.integers(0, len(hull.simplices), 400)
+    bary = rng.dirichlet(np.ones(3), 400)
+    shell = np.einsum('nk,nkd->nd', bary, verts[hull.simplices[f]])
+    shell += hull.equations[f, :3] * rng.uniform(0, 0.01 * np.ptp(verts, axis=0).max(), (400, 1))
+    inner = rng.dirichlet(np.ones(len(verts)), 200) @ verts
+    path = str(tmp_path / os.path.basename(rel))
+    write_mesh(path, np.concatenate([verts, shell, inner]))
     v = cmesh.load_vertices(path)
+    assert len(v) >= len(verts) + 600 and len(ConvexHull(v).vertices) > 64
     V, P = cmesh.reduced_hull(v)
     assert 4 <= len(V) <= 32 and len(P) <= 64
+    assert np.allclose(V.min(axis=0), v.min(axis=0)) and np.allclose(V.max(axis=0), v.max(axis=0))   # the axis extremes are kept
     assert np.allclose(np.linalg.norm(P[:, :3], axis=1), 1.0, atol=1e-9)
     # every reduced vertex is a vertex of the mesh, every one of them satisfies every plane
     assert np.min(np.linalg.norm(v[None, :, :] - V[:, None, :], axis=2), axis=1).max() < 1e-9
