@@ -472,7 +472,88 @@ class TiltTerminal(_OpAddon):
         return self._term.bool()
 
 
+class RaySensor(_OpAddon):
+    """Range finder (pybullet's rayTestBatch): rays from a point on a frame of the parent (or fixed in the world for an
+    environment-level sensor) against the collision shapes of every body, the parent included.  Per ray the distance to the first
+    surface the ray enters with t in (min, max] (max on a miss) and, with `include_hit_object`, the body index hit (load order, as
+    pybullet's uid and the segmentation mask; -1 on a miss).  Cast by dg_ray_kernel after every step / reset / observe (op
+    `RAY_SENSOR`).  Keys: frame (joint name, default the base), xyz, rpy (sensor pose in that frame, the camera's convention), range
+    [min, max], num_rays / horizontal_fov / vertical_angles (a pattern about the sensor's z axis: azimuths k 360 / n over a full
+    turn, else -fov/2 .. +fov/2 inclusive; one layer per elevation in degrees, layer-major) or `directions` (explicit, in the
+    sensor frame, normalised), include_hit_object."""
+    MAX_RAYS = 1024
+
+    def __init__(self, parent, config):
+        super().__init__(parent, config)
+        self.frame_id = -1
+        if 'frame' in config:
+            names = parent.body.joint_names() if _is_model(parent) else []
+            if config.get('frame') not in names:
+                raise ValueError('ray_sensor: unknown frame %r' % (config.get('frame'), ))
+            self.frame_id = parent.get_frame_id(config.get('frame'))
+        self.xyz = [float(v) for v in config.get('xyz', [0.0, 0.0, 0.0])]
+        self.rpy = [float(v) for v in config.get('rpy', [0.0, 0.0, 0.0])]
+        rng = [float(v) for v in config.get('range', [0.0, 10.0])]
+        if len(rng) != 2:
+            raise ValueError('ray_sensor: range must be [min, max]')
+        self.min, self.max = rng
+        if self.min < 0 or self.min >= self.max:
+            raise ValueError('ray_sensor: range needs 0 <= min < max (got %r)' % (rng, ))
+        self.include_hit_object = bool(config.get('include_hit_object', False))
+        if 'directions' in config:
+            d = np.asarray(config.get('directions'), float).reshape(-1, 3)
+            n = np.linalg.norm(d, axis=1)
+            if d.shape[0] < 1 or np.any(n == 0):
+                raise ValueError('ray_sensor: directions must be non-empty and of non-zero length')
+            self.directions = d / n[:, None]
+        else:
+            self.directions = self.pattern(int(config.get('num_rays', 1)), float(config.get('horizontal_fov', 360.0)),
+                                           [float(v) for v in config.get('vertical_angles', [0.0])])
+        self.num_rays = len(self.directions)
+        if self.num_rays > self.MAX_RAYS:
+            raise ValueError('ray_sensor: %d rays, at most %d per sensor' % (self.num_rays, self.MAX_RAYS))
+        self.observation_space = spaces.Dict({'distance': spaces.Box(self.min, self.max, shape=(self.num_rays, ), dtype='float32')})
+        if self.include_hit_object:
+            self.observation_space.spaces['hit_object'] = spaces.Box(-1.0, np.inf, shape=(self.num_rays, ), dtype='float32')
+
+    @staticmethod
+    def pattern(num_rays, horizontal_fov, vertical_angles):
+        """Unit directions of the pattern, layer-major: azimuths about z, one layer per elevation (degrees)."""
+        if num_rays < 1:
+            raise ValueError('ray_sensor: num_rays must be at least 1')
+        if not 0.0 < horizontal_fov <= 360.0:
+            raise ValueError('ray_sensor: horizontal_fov must be in (0, 360]')
+        if len(vertical_angles) < 1:
+            raise ValueError('ray_sensor: vertical_angles needs at least one elevation')
+        k = np.arange(num_rays, dtype=float)
+        if horizontal_fov == 360.0:
+            az = k * 360.0 / num_rays
+        else:
+            az = -horizontal_fov / 2 + k * (horizontal_fov / (num_rays - 1)) if num_rays > 1 else np.zeros(1)
+        az = np.radians(az)
+        out = []
+        for el in np.radians(np.asarray(vertical_angles, float)):
+            out.append(np.stack([np.cos(el) * np.cos(az), np.cos(el) * np.sin(az), np.full_like(az, np.sin(el))], axis=1))
+        return np.concatenate(out, axis=0)
+
+    def compile(self, sb):
+        from ..compiler.mathutil import quat_from_euler
+        frame = self.parent.body.frame(self.frame_id) if _is_model(self.parent) else -1
+        R = self.num_rays
+        self.op = sb.add_op('RAY_SENSOR', [frame, R, int(self.include_hit_object)],
+                            self.xyz + list(quat_from_euler(self.rpy)) + [self.min, self.max] + self.directions.reshape(-1).tolist(),
+                            n_obs=2 * R if self.include_hit_object else R)
+
+    def observe(self):
+        R = self.num_rays
+        out = {'distance': self._obs[:, 0:R]}
+        if self.include_hit_object:
+            out['hit_object'] = self._obs[:, R:2 * R]
+        return out
+
+
 BUILTIN_ADDONS = {
+    'ray_sensor': RaySensor,
     'filtered_link_wrench': FilteredLinkWrench, 'tilt_terminal': TiltTerminal,
     'ik_controller': InverseKinematicsController, 'joint_controller': JointController, 'admittance_controller': AdmittanceController,
     'camera': Camera, 'joint_state_sensor': JointStateSensor, 'object_state_sensor': ObjectStateSensor,

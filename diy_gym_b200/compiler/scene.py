@@ -58,6 +58,10 @@ JOINT_TYPES = {'fixed': 0, 'revolute': 1, 'continuous': 1, 'prismatic': 2}
 OP = dict(JOINT_CTRL=1, EXT_FORCE=2, IK_CTRL=3, JOINT_SENSOR=4, OBJECT_SENSOR=5, REACH_TARGET=6, ELECTRICITY=7,
           STUCK_JOINT=8, TIME_PENALTY=9, EPISODE_TIMER=10, RESPAWN=11, JOINT_RESET=12, DYN_RANDOMIZE=13, ADMITTANCE=14, FT_SENSOR=15,
           FILTERED_WRENCH=16, TILT_TERMINAL=17, VIS_RANDOMIZE=18)
+# Ops evaluated by a kernel of their own after the step launches, which the step kernel and the oracle's step skip (they pass over
+# op codes they do not know).  Their codes continue the numbering above and are defined beside their kernel, not in
+# scene_sections.h: RAY_SENSOR in csrc/dg_ray.cuh (dg_ray_kernel).
+KERNEL_OPS = dict(RAY_SENSOR=19)
 
 # Engine semantics that SURVEY Appendix A could only RECALL (no pybullet here to check): each is a named switch of the scene
 # header, honoured by the kernels and by the oracle alike, so that the day a pybullet golden vector disagrees the fix is a flag.
@@ -190,7 +194,7 @@ class SceneBuilder:
 
     def add_op(self, op, iargs=(), fargs=(), n_act=0, n_obs=0, n_rew=0, n_term=0):
         """Append an add-on op; returns the record so the caller can read the assigned offsets later."""
-        rec = dict(type=OP[op], iargs=[int(v) for v in iargs], fargs=[float(v) for v in fargs], n_act=n_act, n_obs=n_obs,
+        rec = dict(type=OP[op] if op in OP else KERNEL_OPS[op], iargs=[int(v) for v in iargs], fargs=[float(v) for v in fargs], n_act=n_act, n_obs=n_obs,
                    n_rew=n_rew, n_term=n_term)
         self.ops.append(rec)
         return rec

@@ -12,9 +12,11 @@
 #include <string.h>
 
 #include <string>
+#include <vector>
 
 #include "../../include/diygym_b200.h"
 #include "dg_env.cuh"
+#include "dg_ray.cuh"
 
 namespace dg {
 
@@ -341,51 +343,7 @@ __global__ void dg_init_kernel(const __grid_constant__ DevScene sc, float* state
 }
 
 // ---------------------------------------------------------------- camera ----------------------------------------
-// nearest hit of a ray (shape-local origin o, direction dir) within (1e-9, tmax)
-__device__ __forceinline__ bool ray_shape(int type, const float* d, const float* o, const float* dir, float tmax, float* t_out, float* n_out) {
-  float best = tmax; bool hit = false; float nb_[3] = {0, 0, 1};
-  if (type == SHAPE_SPHERE || type == SHAPE_CAPSULE) {
-    int nsph = type == SHAPE_SPHERE ? 1 : 2;
-    for (int s = 0; s < nsph; s++) {
-      float cz = type == SHAPE_SPHERE ? 0.f : (s ? d[1] : -d[1]);
-      float oc[3] = {o[0], o[1], o[2] - cz};
-      float A = v_dot(dir, dir), B = v_dot(oc, dir), Cc = v_dot(oc, oc) - d[0] * d[0], disc = B * B - A * Cc;
-      if (disc < 0) continue;
-      float t = (-B - sqrtf(disc)) / A;
-      if (t > 1e-9f && t < best) { best = t; hit = true; for (int i = 0; i < 3; i++) nb_[i] = (oc[i] + t * dir[i]) / d[0]; }
-    }
-  }
-  if (type == SHAPE_CAPSULE || type == SHAPE_CYLINDER) {
-    float A = dir[0] * dir[0] + dir[1] * dir[1], B = o[0] * dir[0] + o[1] * dir[1], Cc = o[0] * o[0] + o[1] * o[1] - d[0] * d[0];
-    float disc = B * B - A * Cc;
-    if (A > 1e-18f && disc >= 0) {
-      float t = (-B - sqrtf(disc)) / A, z = o[2] + t * dir[2];
-      if (t > 1e-9f && t < best && fabsf(z) <= d[1]) { best = t; hit = true; nb_[0] = (o[0] + t * dir[0]) / d[0]; nb_[1] = (o[1] + t * dir[1]) / d[0]; nb_[2] = 0; }
-    }
-    if (type == SHAPE_CYLINDER && fabsf(dir[2]) > 1e-18f) for (int s = -1; s <= 1; s += 2) {
-      float t = (s * d[1] - o[2]) / dir[2], x = o[0] + t * dir[0], y = o[1] + t * dir[1];
-      if (t > 1e-9f && t < best && x * x + y * y <= d[0] * d[0]) { best = t; hit = true; nb_[0] = 0; nb_[1] = 0; nb_[2] = (float)s; }
-    }
-  }
-  if (type == SHAPE_BOX) {
-    // slab test without branches: the three axes are independent (reciprocals by the SFU, ~1 ulp: the depth tolerance
-    // is 1e-4); a ray parallel to a slab gets (-inf, +inf) inside it and an empty interval outside
-    float t0 = -1e30f, t1 = 1e30f; int ax0 = 0; float sg0 = 1;
-#pragma unroll
-    for (int i = 0; i < 3; i++) {
-      const bool par = fabsf(dir[i]) < 1e-18f, inside = fabsf(o[i]) <= d[i];
-      const float inv = __fdividef(1.0f, par ? 1.0f : dir[i]);
-      const float ua = (-d[i] - o[i]) * inv, ub = (d[i] - o[i]) * inv;
-      float ta = fminf(ua, ub), tb = fmaxf(ua, ub); const float sg = ua > ub ? 1.f : -1.f;
-      ta = par ? (inside ? -1e30f : 1e30f) : ta; tb = par ? (inside ? 1e30f : -1e30f) : tb;
-      if (ta > t0) { t0 = ta; ax0 = i; sg0 = sg; }
-      t1 = fminf(t1, tb);
-    }
-    if (t0 <= t1 && t0 > 1e-9f && t0 < best) { best = t0; hit = true; nb_[0] = ax0 == 0 ? sg0 : 0.f; nb_[1] = ax0 == 1 ? sg0 : 0.f; nb_[2] = ax0 == 2 ? sg0 : 0.f; }
-  }
-  if (hit) { *t_out = best; v_cpy(n_out, nb_); }
-  return hit;
-}
+// (ray_shape, the exact ray-shape test, is in dg_ray.cuh)
 
 // per visual shape in shared memory, in FRONT-TO-BACK order (by the nearest eye-space depth of its oriented bounding box):
 //   R(9) p(3) dims(4) rgb(3) type(1) bound radius(1) | M = R_shape^T R_cam (9), ray origin in the shape frame (3),
@@ -624,6 +582,27 @@ __global__ void __launch_bounds__(256, 3) dg_render_kernel(const __grid_constant
   }
 }
 
+// ---------------------------------------------------------------- ray_sensor ------------------------------------
+// dg_ray_kernel: every ray_sensor op of the scene (dg_ray.cuh) in one launch, one warp per environment.  The warp puts the world
+// poses of the collision shapes that move (from the state row's link cache) into its slice of shared memory; baked shapes use the
+// compiled world poses (DevScene::shape_wb, the same for every environment: L1 / L2 resident).  Lane l casts rays l, l + 32, ...
+// against every shape (bounding-sphere rejection, then the exact test in the shape frame); consecutive lanes store consecutive
+// floats of the op's slice of the observation row.
+constexpr int kRayWarps = 4;   // environments per block
+__global__ void __launch_bounds__(32 * kRayWarps) dg_ray_kernel(const __grid_constant__ DevScene sc, const float* state, float* obs, const uint8_t* mask, int n_envs) {
+  extern __shared__ __align__(16) float ray_mov[];   // [kRayWarps][nshw][12]
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * kRayWarps + warp;
+  if (e >= n_envs || (mask != nullptr && mask[e] == 0)) return;   // (whole warps: no barrier below spans more than one)
+  float* mov = ray_mov + (size_t)warp * 12 * sc.nshw;
+  Env C; C.sc = &sc; C.st = const_cast<float*>(state) + (size_t)e * sc.S; C.obs = obs + (size_t)e * sc.n_obs;
+  C.ws = nullptr; C.wg = nullptr; C.pr = nullptr; C.dbg = nullptr; C.dropped = nullptr; C.rs_used = nullptr; C.no_hot = 0;
+  C.link_i = sc.link_i; C.link_f = sc.link_f; C.link_x = sc.link_x;
+  ray_stage_shapes(C, mov, lane, 32);
+  __syncwarp();
+  ray_env(C, mov, lane, 32);
+}
+
 }  // namespace dg
 
 // ---------------------------------------------------------------- C ABI ------------------------------------------
@@ -662,6 +641,8 @@ struct DgWorld {
   // what separates the step from the sum of its kernels
   int use_graph = 0; cudaStream_t cap = nullptr; cudaGraph_t graph = nullptr; cudaGraphExec_t graph_exec = nullptr;
   unsigned long long graph_key[4] = {0, 0, 0, 0}; bool graph_valid = false;
+  // ray_sensor ops (dg_ray_kernel, launched after the step / reset / observe launches when the scene has any)
+  std::vector<int> ray_ops; size_t ray_smem = 0;
   int64_t launches = 0;
   std::string err;
 };
@@ -824,6 +805,17 @@ int dg_world_create(const int32_t* ibuf, int n_ibuf, const double* fbuf, int n_f
     }
   }
   if (cudaMalloc(&w->dropped, sizeof(unsigned)) != cudaSuccess || cudaMemset(w->dropped, 0, sizeof(unsigned)) != cudaSuccess) { g_create_err = "cudaMalloc of the contact-drop counter failed"; cudaGetLastError(); dg_world_destroy(w); return DG_E_CUDA; }
+  {
+    // ray_sensor ops: which ops, and the shared memory of dg_ray_kernel (the world poses of the moving shapes, per warp)
+    const DevScene& hd = w->hs.dev;   // (host pointers)
+    for (int k = 0; k < hd.nop; k++) if (hd.op_i[DG_OP_I_W * k] == OP_RAY_SENSOR) w->ray_ops.push_back(k);
+    w->ray_smem = (size_t)kRayWarps * 12 * hd.nshw * sizeof(float);
+    if (!w->ray_ops.empty() && w->ray_smem > 48 * 1024) {
+      if (w->ray_smem > smem_cap || cudaFuncSetAttribute(dg_ray_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)w->ray_smem) != cudaSuccess) {
+        g_create_err = "ray_sensor: the moving collision shapes do not fit in shared memory"; cudaGetLastError(); dg_world_destroy(w); return DG_E_NOMEM;
+      }
+    }
+  }
   *out = w;
   return DG_OK;
 }
@@ -906,7 +898,7 @@ int dg_init_state(DgWorld* w, void* stream) {
   return DG_OK;
 }
 
-static int run(DgWorld* w, int mode, const uint8_t* mask, void* stream) {
+static int run_step(DgWorld* w, int mode, const uint8_t* mask, void* stream) {
   if (!w) return DG_E_ARG;
   if (!w->bound) { w->err = "buffers not bound"; return DG_E_UNBOUND; }
   DeviceGuard guard(w->device);
@@ -1009,6 +1001,17 @@ int dg_debug_read(DgWorld* w, unsigned long long* out, int n) {
   CK(w, cudaDeviceSynchronize());
   CK(w, cudaMemcpy(out, w->dbg, (size_t)n * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   CK(w, cudaMemset(w->dbg, 0, (size_t)w->grid * 64 * sizeof(unsigned long long)));
+  return DG_OK;
+}
+// The step / reset / observe launches, then the ray_sensor ops (one launch of dg_ray_kernel on the same stream, after whichever
+// schedule the step took: it reads the link cache the step left in the state rows).  A reset only casts the masked environments' rays.
+static int run(DgWorld* w, int mode, const uint8_t* mask, void* stream) {
+  const int rc = run_step(w, mode, mask, stream);
+  if (rc != DG_OK || w->ray_ops.empty()) return rc;
+  DeviceGuard guard(w->device);
+  w->launches++;
+  dg_ray_kernel<<<(w->n_envs + kRayWarps - 1) / kRayWarps, 32 * kRayWarps, w->ray_smem, (cudaStream_t)stream>>>(w->dev, w->buf.state, w->buf.obs, mode == 1 ? mask : nullptr, w->n_envs);
+  CK(w, cudaGetLastError());
   return DG_OK;
 }
 int dg_step(DgWorld* w, void* stream) { return run(w, 0, nullptr, stream); }

@@ -77,7 +77,9 @@ int dg_set_action_mask(DgWorld* w, const uint8_t* op_enabled, int n_ops);
 int dg_init_state(DgWorld* w, void* stream);
 
 /* One DIYGym.step for every environment: add-on update(action) -> stepSimulation -> observe/reward/is_terminal.
- * Replaces /root/reference/diy_gym/diy_gym.py:187-209 (p.stepSimulation at :207 and every add-on hook it fans out to). */
+ * Replaces /root/reference/diy_gym/diy_gym.py:187-209 (p.stepSimulation at :207 and every add-on hook it fans out to).
+ * Scenes with ray_sensor add-ons: their distances (and hit body ids) are part of obs, cast by one more launch on `stream`
+ * after the step (dg_ray_kernel); the same holds for dg_reset (masked environments only), dg_observe and dg_step_host. */
 int dg_step(DgWorld* w, void* stream);
 /* Measurement aid (no reference counterpart): per-block, per-phase cycle sums of the step kernel.  enable != 0 allocates and
  * clears a [grid][64] table keyed by (source line of the phase in dg_env.cuh) & 63; dg_debug_read copies n <= grid * 64
@@ -85,10 +87,11 @@ int dg_step(DgWorld* w, void* stream);
 int dg_debug_phase_cycles(DgWorld* w, int enable);
 int dg_debug_read(DgWorld* w, unsigned long long* out, int n);
 /* DIYGym.reset for the environments whose mask byte is non-zero (mask_dev == NULL: all).
- * Replaces /root/reference/diy_gym/diy_gym.py:130-148 (add-on reset hooks, hot-start steps, observe). */
+ * Replaces /root/reference/diy_gym/diy_gym.py:130-148 (add-on reset hooks, hot-start steps, observe).  Ray_sensor rays of the
+ * masked environments are cast after it (see dg_step); the other environments' obs rows are not touched. */
 int dg_reset(DgWorld* w, const uint8_t* mask_dev, void* stream);
 /* DIYGym.observe / reward / is_terminal on the state rows as they are (no physics): refreshes the link-pose cache the sensors
- * read and evaluates every sensor / reward / terminal op into obs / reward / term.
+ * read and evaluates every sensor / reward / terminal op into obs / reward / term (ray_sensor rays included, see dg_step).
  * Replaces /root/reference/diy_gym/diy_gym.py:211-222 (observe, reward, is_terminal -> walk_addons). */
 int dg_observe(DgWorld* w, void* stream);
 /* Camera add-on number `cam`: rgb [n_envs][H][W][3] float in [0,1], depth [n_envs][H][W] eye-space z (negative).
