@@ -19,6 +19,8 @@ class DgBufferTable(ctypes.Structure):
                 ('reward', ctypes.c_void_p), ('term', ctypes.c_void_p)]
 
 
+DYN_MAX_N = 64   # DG_DYN_MAX_N of include/diygym_b200.h: largest number of generalized coordinates dg_body_dynamics accepts
+
 Q = dict(STATE_SIZE=0, PARAM_SIZE=1, N_ACT=2, N_OBS=3, N_REW=4, N_TERM=5, N_ENVS=6, TEAM=7, BLOCK_THREADS=8, GRID_BLOCKS=9,
          SMEM_BYTES=10, WS_FLOATS=11, N_CAMERAS=12, LAUNCHES=13, RS_ASHARED=14, SOLVER=15, MAX_CONTACTS=16, CONTACTS_DROPPED=17, SPLIT=18)
 
@@ -63,6 +65,8 @@ def load_library():
     L.dg_debug_phase_cycles.argtypes = [vp, ctypes.c_int]
     L.dg_debug_read.restype = ctypes.c_int
     L.dg_debug_read.argtypes = [vp, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
+    L.dg_body_dynamics.restype = ctypes.c_int
+    L.dg_body_dynamics.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_float), vp, vp, vp, vp, vp, vp, vp]
     L.dg_measure_fp32_peak.restype = ctypes.c_int
     L.dg_measure_fp32_peak.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_double)]
     _lib = L
@@ -191,6 +195,20 @@ class World:
         """Host-buffer step: numpy (ideally pinned) in, numpy out, synchronous."""
         p = lambda a: ctypes.c_void_p(a.ctypes.data) if a is not None and a.size else None
         self._check(self.L.dg_step_host(self._h, p(action_host), p(obs_host), p(reward_host), p(term_host), self._stream()))
+
+    def body_dynamics(self, body, link=-1, point=(0., 0., 0.), q=None, qd=None, qdd=None, jac=False, mass=False, tau=False):
+        """Jacobian [N, 6, n] (linear rows first), mass matrix [N, n, n] and inverse dynamics [N, n] of body `body` (dg_body_dynamics):
+        new tensors, None where not asked for.  q [N, n_dof], qd / qdd [N, n]: contiguous float32 tensors on this world's device or
+        None (the state row's q, the state row's velocities, zero).  Asynchronous on the current stream."""
+        b = self.scene.bodies[body]
+        n, N, dev = b.n_dofs + (6 if b.kind == 2 else 0), self.n_envs, self.device
+        outs = [torch.empty((N, 6, n), dtype=torch.float32, device=dev) if jac else None,
+                torch.empty((N, n, n), dtype=torch.float32, device=dev) if mass else None,
+                torch.empty((N, n), dtype=torch.float32, device=dev) if tau else None]
+        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        pt = (ctypes.c_float * 3)(*[float(x) for x in point])
+        self._check(self.L.dg_body_dynamics(self._h, int(body), int(link), pt, p(q), p(qd), p(qdd), *[p(o) for o in outs], self._stream()))
+        return tuple(outs)
 
     # named views into the state / parameter rows (same names as csrc/scene_sections.h)
     def s(self, name, n):

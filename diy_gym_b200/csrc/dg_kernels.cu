@@ -17,6 +17,7 @@
 #include "../../include/diygym_b200.h"
 #include "dg_env.cuh"
 #include "dg_ray.cuh"
+#include "dg_dyn.cuh"
 
 namespace dg {
 
@@ -603,6 +604,27 @@ __global__ void __launch_bounds__(32 * kRayWarps) dg_ray_kernel(const __grid_con
   ray_env(C, mov, lane, 32);
 }
 
+// ---------------------------------------------------------------- dynamics queries --------------------------------
+// dg_dyn_kernel: Jacobian / mass matrix / inverse dynamics of one body (dg_dyn.cuh), one warp per environment.  Lane 0 walks the
+// body's links once (poses, velocities, accelerations) into the warp's slice of shared memory; then the lanes split the links
+// (world inertias, link wrenches) and the outputs (Jacobian columns, upper-triangle entries of M, generalized forces).
+constexpr int kDynWarps = 4;   // environments per block
+__global__ void __launch_bounds__(32 * kDynWarps) dg_dyn_kernel(const __grid_constant__ DevScene sc, const DynArgs a, const float* state, const float* param, int n_envs) {
+  extern __shared__ __align__(16) float dyn_smem[];   // [kDynWarps][dyn_scratch_floats(nl, n)]
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * kDynWarps + warp;
+  if (e >= n_envs) return;   // (whole warps: no barrier below spans more than one)
+  float* base = dyn_smem + (size_t)warp * dyn_scratch_floats(a.nl, a.n);
+  unsigned long long* msk = reinterpret_cast<unsigned long long*>(base);
+  float* L = base + 2 * a.nl; float* col = L + DL_W_ * a.nl; float* pt = col + DC_W_ * a.n;
+  const float* pr = param + (size_t)e * sc.P;
+  if (lane == 0) dyn_chain(sc, a, state + (size_t)e * sc.S, pr, e, msk, L, col);
+  __syncwarp();
+  dyn_links(sc, a, pr, L, pt, lane, 32);
+  __syncwarp();
+  dyn_outputs(a, e, msk, L, col, pt, lane, 32);
+}
+
 }  // namespace dg
 
 // ---------------------------------------------------------------- C ABI ------------------------------------------
@@ -1015,6 +1037,30 @@ static int run(DgWorld* w, int mode, const uint8_t* mask, void* stream) {
   return DG_OK;
 }
 int dg_step(DgWorld* w, void* stream) { return run(w, 0, nullptr, stream); }
+
+int dg_body_dynamics(DgWorld* w, int body, int link, const float point[3], const float* q_dev, const float* qd_dev, const float* qdd_dev,
+                     float* jac_dev, float* mass_dev, float* tau_dev, void* stream) {
+  if (!w) return DG_E_ARG;
+  if (!w->bound) { w->err = "dg_body_dynamics: buffers not bound"; return DG_E_UNBOUND; }
+  const DevScene& hd = w->hs.dev;   // (host pointers)
+  if (body < 0 || body >= hd.nb) { w->err = "dg_body_dynamics: no such body"; return DG_E_ARG; }
+  const int* bi = hd.body_i + DG_BODY_I_W * body;
+  DynArgs a;
+  a.body = body; a.link = link; a.n = (bi[0] == 2 ? 6 : 0) + bi[4]; a.nl = bi[2] + 1;
+  if (bi[0] == 0 || a.n == 0) { w->err = "dg_body_dynamics: the body has no degrees of freedom"; return DG_E_ARG; }
+  if (a.n > DG_DYN_MAXN) { w->err = "dg_body_dynamics: the body has " + std::to_string(a.n) + " generalized coordinates, more than " + std::to_string((int)DG_DYN_MAXN); return DG_E_ARG; }
+  if (link < -1 || link >= bi[2]) { w->err = "dg_body_dynamics: no such link"; return DG_E_ARG; }
+  for (int i = 0; i < 3; i++) a.point[i] = point ? point[i] : 0.f;
+  a.q = q_dev; a.qd = qd_dev; a.qdd = qdd_dev; a.jac = jac_dev; a.mass = mass_dev; a.tau = tau_dev;
+  if (!jac_dev && !mass_dev && !tau_dev) return DG_OK;
+  DeviceGuard guard(w->device);
+  const size_t smem = (size_t)kDynWarps * dyn_scratch_floats(a.nl, a.n) * sizeof(float);
+  if (smem > 48 * 1024) CK(w, cudaFuncSetAttribute(dg_dyn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  w->launches++;
+  dg_dyn_kernel<<<(w->n_envs + kDynWarps - 1) / kDynWarps, 32 * kDynWarps, smem, (cudaStream_t)stream>>>(w->dev, a, w->buf.state, w->buf.param, w->n_envs);
+  CK(w, cudaGetLastError());
+  return DG_OK;
+}
 int dg_reset(DgWorld* w, const uint8_t* mask_dev, void* stream) { return run(w, 1, mask_dev, stream); }
 int dg_observe(DgWorld* w, void* stream) { return run(w, 2, nullptr, stream); }
 

@@ -15,6 +15,7 @@ import torch
 from . import torch_math as tm
 from .addons.addon import AddonFactory, Receptor
 from .assets import resolve_model
+from .backend import DYN_MAX_N
 from .compiler.mathutil import quat_from_euler
 
 
@@ -140,3 +141,69 @@ class Model(Receptor):
             torque = tm.quat_rotate(self.link_state(link)[1], torque)
         o_t = self._h('S_EXTT') + 3 * f
         st[:, o_t:o_t + 3] += torque
+
+    def apply_joint_torque(self, joint_ids, torque):
+        """Batched setJointMotorControlArray(TORQUE_CONTROL): adds torque [N, len(joint_ids)] (or anything that broadcasts to it)
+        to the applied joint torque of those movable joints; acts during the next step only, like apply_external_force."""
+        cols = self._dofs(joint_ids, 'apply_joint_torque')
+        st = self.world.state
+        try:
+            torque = torch.as_tensor(torque, device=st.device, dtype=torch.float32).expand(st.shape[0], len(cols))
+        except RuntimeError as e:
+            raise ValueError('apply_joint_torque: torque must broadcast to [%d, %d] (%s)' % (st.shape[0], len(cols), e))
+        st.index_add_(1, torch.as_tensor(cols, device=st.device) + self._h('S_JTORQUE'), torque)
+
+    def disable_motors(self, joint_ids):
+        """setJointMotorControlArray(VELOCITY_CONTROL, forces=0): switches off the default velocity motor of those movable joints
+        in every environment (the scene's default state).  Constructor-time only: call it from an add-on's __init__."""
+        dofs = self._dofs(joint_ids, 'disable_motors')
+        if self.env.builder.finalized is not None:
+            raise ValueError('disable_motors: the scene is already compiled; call it from an add-on constructor')
+        self.env.builder.motors_off += dofs
+
+    def _dofs(self, joint_ids, what):
+        ids, movable = list(joint_ids), set(self.body.movable_joints())
+        bad = [i for i in ids if i not in movable]
+        if bad:
+            raise ValueError('%s: joints %s of %s are not movable joints (fixed or unknown)' % (what, bad, self.name))
+        return [self.body.global_dof(i) for i in ids]
+
+    # ---- rigid-body dynamics queries (dg_body_dynamics) ----------------------------------------------
+    # Generalized velocity nu: [omega_base (world), v_base (world, base COM), qd] for a floating base, qd for a fixed one, with qd
+    # in movable_joints() order; n = len(nu).  q [N, n_dof] holds joint positions only: the base pose is the state row's.
+    def jacobian(self, frame_id=-1, local_position=(0., 0., 0.), q=None):
+        """calculateJacobian: (J_lin [N, 3, n], J_ang [N, 3, n]) in world axes of the point `local_position`, given in the COM frame
+        of link `frame_id` (-1 = base), at joint positions q (None: the state's)."""
+        if not -1 <= int(frame_id) < self.num_joints():
+            raise ValueError('jacobian: frame %d out of range [-1, %d)' % (frame_id, self.num_joints()))
+        p = [float(x) for x in np.asarray(local_position, float).reshape(-1)]
+        if len(p) != 3:
+            raise ValueError('jacobian: local_position needs 3 entries')
+        J = self._dynamics(int(frame_id), p, q, None, None, jac=True)[0]
+        return J[:, :3], J[:, 3:]
+
+    def mass_matrix(self, q=None):
+        """calculateMassMatrix: M [N, n, n] at joint positions q (None: the state's); masses and inertias of the parameter row."""
+        return self._dynamics(-1, (0., 0., 0.), q, None, None, mass=True)[1]
+
+    def inverse_dynamics(self, q=None, qd=None, qdd=None):
+        """calculateInverseDynamics: tau [N, n] = M(q) qdd + C(q, nu) nu + G(q) with the scene's gravity (None: the state's q, the
+        state's nu, zero qdd).  For a floating base tau[:, :6] is the base wrench [torque about the base COM, force], world axes.
+        Joint damping, motors, limits and contacts are not included."""
+        return self._dynamics(-1, (0., 0., 0.), q, qd, qdd, tau=True)[2]
+
+    def _dynamics(self, link, point, q, qd, qdd, jac=False, mass=False, tau=False):
+        n = self.body.n_dofs + (6 if self.body.kind == 2 else 0)
+        if n == 0:
+            raise ValueError('%s has no degrees of freedom: no dynamics to query' % self.name)
+        if n > DYN_MAX_N:
+            raise ValueError('%s has %d generalized coordinates; the dynamics queries take at most %d' % (self.name, n, DYN_MAX_N))
+        st = self.world.state
+        args = []
+        for name, t, width in (('q', q, self.body.n_dofs), ('qd', qd, n), ('qdd', qdd, n)):
+            if t is not None:
+                if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or t.device != st.device or tuple(t.shape) != (st.shape[0], width):
+                    raise ValueError('%s must be a float32 tensor of shape [%d, %d] on %s' % (name, st.shape[0], width, st.device))
+                t = t.contiguous()
+            args.append(t)
+        return self.world.body_dynamics(self.uid, link, point, *args, jac=jac, mass=mass, tau=tau)

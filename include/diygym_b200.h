@@ -104,6 +104,22 @@ int dg_render_seg(DgWorld* w, int cam, float* rgb_dev, float* depth_dev, float* 
  * which the reference divides by 255 (sensors/camera.py:76-78); a quarter of the colour bytes to move.  seg_dev may be NULL. */
 int dg_render_u8(DgWorld* w, int cam, uint8_t* rgb_dev, float* depth_dev, float* seg_dev, void* stream);
 
+/* Rigid-body dynamics of body `body` (load order) for every environment, from its state and parameter rows: one launch on `stream`.
+ * Generalized velocity nu: [omega_base, v_base (world axes, base COM), qd] for a floating base, qd for a fixed one; n = len(nu) <=
+ * DG_DYN_MAX_N.  q_dev [n_envs][n_dof] joint positions (the base pose always comes from the state row), qd_dev / qdd_dev
+ * [n_envs][n]; NULL: the state row's q, the state row's nu, zero.  Outputs, NULL = not computed:
+ *   jac_dev  [n_envs][6][n]  Jacobian of the point `point` (link COM frame; NULL = the COM) of link `link` (-1 = base), world axes,
+ *                            linear rows first (p.calculateJacobian)
+ *   mass_dev [n_envs][n][n]  M(q) (p.calculateMassMatrix)
+ *   tau_dev  [n_envs][n]     M(q) qdd + C(q, nu) nu + G(q), the scene's gravity; a floating base's first six entries are the base
+ *                            wrench [torque about the base COM, force] (p.calculateInverseDynamics)
+ * Masses and inertias are the parameter row's (dynamics_randomizer is honoured); joint damping, motors, limits, contacts and welds
+ * are not part of it.  Writes nothing but the outputs.  DG_E_ARG for a body without degrees of freedom, n > DG_DYN_MAX_N or a
+ * link out of range. */
+enum { DG_DYN_MAX_N = 64 };
+int dg_body_dynamics(DgWorld* w, int body, int link, const float point[3], const float* q_dev, const float* qd_dev, const float* qdd_dev,
+                     float* jac_dev, float* mass_dev, float* tau_dev, void* stream);
+
 /* Host-buffer form of dg_step (the reference-facing call when the caller keeps numpy arrays): copies the actions
  * host->device, steps, copies obs / reward / terminal device->host and waits.  Any output pointer may be NULL. */
 int dg_step_host(DgWorld* w, const float* action_host, float* obs_host, float* reward_host, uint8_t* term_host, void* stream);
