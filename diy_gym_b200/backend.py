@@ -20,6 +20,7 @@ class DgBufferTable(ctypes.Structure):
 
 
 DYN_MAX_N = 64   # DG_DYN_MAX_N of include/diygym_b200.h: largest number of generalized coordinates dg_body_dynamics accepts
+IK_MAX_ND = 64   # DG_IK_MAX_ND of include/diygym_b200.h: largest number of DoF dg_body_ik accepts
 
 Q = dict(STATE_SIZE=0, PARAM_SIZE=1, N_ACT=2, N_OBS=3, N_REW=4, N_TERM=5, N_ENVS=6, TEAM=7, BLOCK_THREADS=8, GRID_BLOCKS=9,
          SMEM_BYTES=10, WS_FLOATS=11, N_CAMERAS=12, LAUNCHES=13, RS_ASHARED=14, SOLVER=15, MAX_CONTACTS=16, CONTACTS_DROPPED=17, SPLIT=18)
@@ -67,6 +68,8 @@ def load_library():
     L.dg_debug_read.argtypes = [vp, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
     L.dg_body_dynamics.restype = ctypes.c_int
     L.dg_body_dynamics.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_float), vp, vp, vp, vp, vp, vp, vp]
+    L.dg_body_ik.restype = ctypes.c_int
+    L.dg_body_ik.argtypes = [vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, ctypes.c_int, ctypes.c_float, vp, vp, vp]
     L.dg_measure_fp32_peak.restype = ctypes.c_int
     L.dg_measure_fp32_peak.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_double)]
     _lib = L
@@ -209,6 +212,18 @@ class World:
         pt = (ctypes.c_float * 3)(*[float(x) for x in point])
         self._check(self.L.dg_body_dynamics(self._h, int(body), int(link), pt, p(q), p(qd), p(qdd), *[p(o) for o in outs], self._stream()))
         return tuple(outs)
+
+    def body_ik(self, body, link, target_pos, target_orn=None, q=None, limits=None, max_iters=20, threshold=1e-4, err=False):
+        """Inverse kinematics of body `body` for link `link` (dg_body_ik): new tensors (q [N, n_dof], err [N, 2] or None).
+        target_pos [N, 3], target_orn [N, 4] or None, q [N, n_dof] or None (the state row's), limits [N, 4, n_dof] or None (no
+        null-space term): contiguous float32 tensors on this world's device.  Asynchronous on the current stream."""
+        nd, N, dev = self.scene.bodies[body].n_dofs, self.n_envs, self.device
+        q_out = torch.empty((N, nd), dtype=torch.float32, device=dev)
+        e = torch.empty((N, 2), dtype=torch.float32, device=dev) if err else None
+        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        self._check(self.L.dg_body_ik(self._h, int(body), int(link), p(target_pos), p(target_orn), p(q), p(limits), int(max_iters),
+                                      float(threshold), p(q_out), p(e), self._stream()))
+        return q_out, e
 
     # named views into the state / parameter rows (same names as csrc/scene_sections.h)
     def s(self, name, n):

@@ -13,7 +13,7 @@ LIB = os.environ.get('DG_LIB') or os.path.join(HERE, 'libdiygym_b200.so')   # DG
 OBJ_DIR = os.path.join(HERE, '_obj')
 SOURCE = 'dg_kernels.cu'
 TEAMS = [1, 2, 4, 8, 16, 32]
-DEPS = ['dg_kernels.cu', 'dg_env.cuh', 'dg_ray.cuh', 'dg_dyn.cuh', 'dg_math.cuh', 'dg_scene.h', 'scene_sections.h', os.path.join('..', '..', 'include', 'diygym_b200.h')]
+DEPS = ['dg_kernels.cu', 'dg_env.cuh', 'dg_ray.cuh', 'dg_dyn.cuh', 'dg_ik.cuh', 'dg_math.cuh', 'dg_scene.h', 'scene_sections.h', os.path.join('..', '..', 'include', 'diygym_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '-Xcompiler', '-fPIC']
 
 

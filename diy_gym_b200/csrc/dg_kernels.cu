@@ -18,6 +18,7 @@
 #include "dg_env.cuh"
 #include "dg_ray.cuh"
 #include "dg_dyn.cuh"
+#include "dg_ik.cuh"
 
 namespace dg {
 
@@ -625,6 +626,41 @@ __global__ void __launch_bounds__(32 * kDynWarps) dg_dyn_kernel(const __grid_con
   dyn_outputs(a, e, msk, L, col, pt, lane, 32);
 }
 
+// ---------------------------------------------------------------- inverse-kinematics query -------------------------
+// dg_ik_kernel: calculateInverseKinematics of one body (dg_ik.cuh), one lane per environment.  Every iteration of the solve walks
+// the link chain serially, so a warp per environment would leave 31 lanes idle; small blocks spread the environments over the
+// SMs.  The block first stages the link tables in shared memory, because ik_solve* and joint_xform read them through shc().
+// MAXD > 0: ik_solve_fast<MAXD, M>, its scratch in a per-thread array; MAXD = 0: the generic ik_solve, its scratch in the world's
+// IK buffer behind the seed record.
+constexpr int kIkThreads = 64;
+template <int MAXD, int M>
+__global__ void __launch_bounds__(kIkThreads) dg_ik_kernel(const __grid_constant__ DevScene sc, const IkArgs a, const float* state, int n_envs) {
+  extern __shared__ __align__(16) float ik_smem[];
+  int* s_link_i = reinterpret_cast<int*>(ik_smem);
+  float* s_link_f = reinterpret_cast<float*>(s_link_i + ((DG_LINK_I_W * sc.nl + 3) & ~3));
+  float* s_link_x = s_link_f + DG_LINK_F_W * sc.nl;
+  for (int i = threadIdx.x; i < DG_LINK_I_W * sc.nl; i += blockDim.x) s_link_i[i] = sc.link_i[i];
+  for (int i = threadIdx.x; i < DG_LINK_F_W * sc.nl; i += blockDim.x) s_link_f[i] = sc.link_f[i];
+  for (int i = threadIdx.x; i < 16 * sc.nl; i += blockDim.x) s_link_x[i] = sc.link_x[i];
+  __syncthreads();
+  const int e = blockIdx.x * kIkThreads + threadIdx.x;
+  if (e >= n_envs) return;
+  Env C;
+  C.sc = &sc; C.link_i = s_link_i; C.link_f = s_link_f; C.link_x = s_link_x;
+  C.st = a.rec + (size_t)e * a.rec_stride;
+  float scr[IkFastScratch<MAXD>::floats];
+  ik_env<MAXD, M>(C, a, state + (size_t)e * sc.S, e, scr);
+}
+template <int MAXD, int M>
+static cudaError_t ik_launch(const DevScene& d, const IkArgs& a, const float* state, int n_envs, size_t smem, cudaStream_t stream) {
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(dg_ik_kernel<MAXD, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  dg_ik_kernel<MAXD, M><<<(n_envs + kIkThreads - 1) / kIkThreads, kIkThreads, smem, stream>>>(d, a, state, n_envs);
+  return cudaGetLastError();
+}
+
 }  // namespace dg
 
 // ---------------------------------------------------------------- C ABI ------------------------------------------
@@ -665,6 +701,8 @@ struct DgWorld {
   unsigned long long graph_key[4] = {0, 0, 0, 0}; bool graph_valid = false;
   // ray_sensor ops (dg_ray_kernel, launched after the step / reset / observe launches when the scene has any)
   std::vector<int> ray_ops; size_t ray_smem = 0;
+  // dg_body_ik: [n_envs][seed record + ik_stride] (dg_ik.cuh), allocated by the first call
+  float* ik_rec = nullptr;
   int64_t launches = 0;
   std::string err;
 };
@@ -853,6 +891,7 @@ void dg_world_destroy(DgWorld* w) {
   if (w->carry) cudaFree(w->carry);
   if (w->rs_lists) cudaFree(w->rs_lists);
   if (w->rs_counts) cudaFree(w->rs_counts);
+  if (w->ik_rec) cudaFree(w->ik_rec);
   if (w->aux) cudaStreamDestroy(w->aux);
   if (w->aux2) cudaStreamDestroy(w->aux2);
   if (w->ev_join2) cudaEventDestroy(w->ev_join2);
@@ -1059,6 +1098,39 @@ int dg_body_dynamics(DgWorld* w, int body, int link, const float point[3], const
   w->launches++;
   dg_dyn_kernel<<<(w->n_envs + kDynWarps - 1) / kDynWarps, 32 * kDynWarps, smem, (cudaStream_t)stream>>>(w->dev, a, w->buf.state, w->buf.param, w->n_envs);
   CK(w, cudaGetLastError());
+  return DG_OK;
+}
+
+int dg_body_ik(DgWorld* w, int body, int link, const float* target_pos_dev, const float* target_orn_dev, const float* q0_dev,
+               const float* limits_dev, int max_iters, float threshold, float* q_out_dev, float* err_dev, void* stream) {
+  if (!w) return DG_E_ARG;
+  if (!w->bound) { w->err = "dg_body_ik: buffers not bound"; return DG_E_UNBOUND; }
+  const DevScene& hd = w->hs.dev;   // (host pointers)
+  if (body < 0 || body >= hd.nb) { w->err = "dg_body_ik: no such body"; return DG_E_ARG; }
+  const int* bi = hd.body_i + DG_BODY_I_W * body;
+  const int ndb = bi[4];
+  if (bi[0] == 0 || ndb == 0) { w->err = "dg_body_ik: the body has no degrees of freedom"; return DG_E_ARG; }
+  if (ndb > DG_IK_MAX_ND) { w->err = "dg_body_ik: the body has " + std::to_string(ndb) + " degrees of freedom, more than " + std::to_string((int)DG_IK_MAX_ND); return DG_E_ARG; }
+  if (link < 0 || link >= bi[2]) { w->err = "dg_body_ik: no such link"; return DG_E_ARG; }
+  if (max_iters < 1) { w->err = "dg_body_ik: max_iters must be at least 1"; return DG_E_ARG; }
+  if (!(threshold >= 0.f)) { w->err = "dg_body_ik: threshold must be a number >= 0"; return DG_E_ARG; }
+  if (!target_pos_dev || !q_out_dev) { w->err = "dg_body_ik: target_pos and q_out are required"; return DG_E_ARG; }
+  DevScene d = w->dev;   // (device pointers)
+  IkArgs a;
+  a.body = body; a.link = bi[1] + link; a.use_orn = target_orn_dev != nullptr;
+  a.s_q = DG_SO(&d, S_Q); a.s_bpos = DG_SO(&d, S_BPOS); a.s_bquat = DG_SO(&d, S_BQUAT);
+  a.seed_floats = ik_scene(d, max_iters, threshold);
+  a.rec_stride = a.seed_floats + d.ik_stride;
+  a.tpos = target_pos_dev; a.torn = target_orn_dev; a.q0 = q0_dev; a.lim = limits_dev; a.q_out = q_out_dev; a.err = err_dev;
+  DeviceGuard guard(w->device);
+  if (!w->ik_rec) CK(w, cudaMalloc(&w->ik_rec, (size_t)w->n_envs * a.rec_stride * sizeof(float)));
+  a.rec = w->ik_rec;
+  const size_t smem = (size_t)(((DG_LINK_I_W * d.nl + 3) & ~3) + (DG_LINK_F_W + 16) * d.nl) * sizeof(float);
+  const cudaStream_t s = (cudaStream_t)stream;
+  // the split of ik_solve_any: register-resident solves up to 12 DoF, the generic one above
+  auto launch = ndb <= 6 ? (a.use_orn ? ik_launch<6, 6> : ik_launch<6, 3>) : ndb <= 12 ? (a.use_orn ? ik_launch<12, 6> : ik_launch<12, 3>) : ik_launch<0, 0>;
+  w->launches++;
+  CK(w, launch(d, a, w->buf.state, w->n_envs, smem, s));
   return DG_OK;
 }
 int dg_reset(DgWorld* w, const uint8_t* mask_dev, void* stream) { return run(w, 1, mask_dev, stream); }

@@ -15,7 +15,7 @@ import torch
 from . import torch_math as tm
 from .addons.addon import AddonFactory, Receptor
 from .assets import resolve_model
-from .backend import DYN_MAX_N
+from .backend import DYN_MAX_N, IK_MAX_ND
 from .compiler.mathutil import quat_from_euler
 
 
@@ -207,3 +207,76 @@ class Model(Receptor):
                 t = t.contiguous()
             args.append(t)
         return self.world.body_dynamics(self.uid, link, point, *args, jac=jac, mass=mass, tau=tau)
+
+    # ---- inverse kinematics (dg_body_ik) and position motors -------------------------------------------
+    def inverse_kinematics(self, frame_id, target_position, target_orientation=None, q=None, lower_limits=None, upper_limits=None,
+                           joint_ranges=None, rest_poses=None, max_iterations=None, residual_threshold=None, return_error=False):
+        """calculateInverseKinematics for every environment: q [N, n_dof] (movable_joints() order) that brings the URDF frame of
+        link `frame_id` to target_position ([N, 3] or [3], world) and, if given, target_orientation ([N, 4] or [4], xyzw, world;
+        None: position only).  The ik_controller op's damped least squares, in the coordinates of the base, whose pose is the
+        state's and stays fixed: from the seed q ([N, n_dof]; None: the state's q), at most max_iterations iterations (None: the
+        scene's ik_iters) while the position residual exceeds residual_threshold (None: the scene's ik_threshold).
+        lower_limits, upper_limits, joint_ranges, rest_poses ([n_dof] or [N, n_dof]): all four add the null-space term; giving
+        only some, or lists of another length, raises ValueError (pybullet silently solves without the term then).
+        return_error=True returns (q, err): err [N, 2] is the link frame's distance from the target (m) and the angle of the
+        remaining rotation (rad, 0 without an orientation) at the returned q.  Inputs are float32 tensors on the world's device;
+        nothing waits for the GPU."""
+        if not 0 <= int(frame_id) < self.num_joints():
+            raise ValueError('inverse_kinematics: frame %d out of range [0, %d): the target must be a link' % (frame_id, self.num_joints()))
+        nd = self.body.n_dofs
+        if nd == 0:
+            raise ValueError('%s has no degrees of freedom: nothing to solve for' % self.name)
+        if nd > IK_MAX_ND:
+            raise ValueError('%s has %d degrees of freedom; inverse_kinematics takes at most %d' % (self.name, nd, IK_MAX_ND))
+        sc = self.env.scene
+        iters = sc.hdr['ik_iters'] if max_iterations is None else max_iterations
+        thr = sc.hdr_f['ik_threshold'] if residual_threshold is None else residual_threshold
+        if int(iters) != iters or iters < 1:
+            raise ValueError('inverse_kinematics: max_iterations must be an integer >= 1, got %r' % (iters, ))
+        if not float(thr) >= 0:
+            raise ValueError('inverse_kinematics: residual_threshold must be >= 0, got %r' % (thr, ))
+        tpos = self._batched('target_position', target_position, 3)
+        torn = None if target_orientation is None else self._batched('target_orientation', target_orientation, 4)
+        if q is not None:
+            q = self._batched('q', q, nd, single=False)
+        lists = (('lower_limits', lower_limits), ('upper_limits', upper_limits), ('joint_ranges', joint_ranges), ('rest_poses', rest_poses))
+        given = [v is not None for _, v in lists]
+        lim = None
+        if any(given):
+            if not all(given):
+                raise ValueError('inverse_kinematics: give all of lower_limits, upper_limits, joint_ranges and rest_poses, or none')
+            lim = torch.stack([self._batched(name, v, nd) for name, v in lists], 1).contiguous()
+        q_out, err = self.world.body_ik(self.uid, int(frame_id), tpos, torn, q, lim, int(iters), float(thr), bool(return_error))
+        return (q_out, err) if return_error else q_out
+
+    def _batched(self, name, t, width, single=True):
+        """t as a contiguous [N, width] tensor: a float32 tensor on the world's device of shape [N, width] (or [width] if single)."""
+        st = self.world.state
+        N = st.shape[0]
+        shapes = [(N, width)] + ([(width, )] if single else [])
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or t.device != st.device or tuple(t.shape) not in shapes:
+            raise ValueError('%s must be a float32 tensor of shape %s on %s' % (name, ' or '.join(str(list(s)) for s in shapes), st.device))
+        return t.expand(N, width).contiguous()
+
+    def set_position_targets(self, joint_ids, target, position_gain=0.03, velocity_gain=1.0, max_force=None):
+        """setJointMotorControlArray(POSITION_CONTROL): the motors of those movable joints drive them to target with the gains
+        position_gain (on the position error) and velocity_gain (on the velocity error, target velocity 0), with at most max_force
+        (None: the URDF effort of each joint, as joint_controller).  Each value is a scalar or broadcasts to
+        [N, len(joint_ids)].  These are the motor fields the joint_controller op writes in position mode.  Like pybullet's motor
+        settings they persist until changed: reset() does not restore them, and a built-in controller op on the same joints
+        overwrites them during the step (ops run inside the kernel, after update())."""
+        ids = list(joint_ids)
+        st = self.world.state
+        cols = torch.as_tensor(self._dofs(ids, 'set_position_targets'), device=st.device)
+        if max_force is None:
+            max_force = [self.body.joint_info(i)['max_force'] for i in ids]
+        vals = []
+        for name, field, v in (('target', 'S_MTPOS', target), ('position_gain', 'S_MKP', position_gain),
+                               ('velocity_gain', 'S_MKD', velocity_gain), ('max_force', 'S_MMAXF', max_force)):
+            try:
+                vals.append((field, torch.as_tensor(v, device=st.device, dtype=torch.float32).expand(st.shape[0], len(ids))))
+            except RuntimeError as e:
+                raise ValueError('set_position_targets: %s must broadcast to [%d, %d] (%s)' % (name, st.shape[0], len(ids), e))
+        for field, v in vals:
+            st[:, cols + self._h(field)] = v
+        st[:, cols + self._h('S_MTVEL')] = 0.0

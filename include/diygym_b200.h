@@ -120,6 +120,24 @@ enum { DG_DYN_MAX_N = 64 };
 int dg_body_dynamics(DgWorld* w, int body, int link, const float point[3], const float* q_dev, const float* qd_dev, const float* qdd_dev,
                      float* jac_dev, float* mass_dev, float* tau_dev, void* stream);
 
+/* Inverse kinematics of body `body` (load order) for every environment (p.calculateInverseKinematics): one launch on `stream`.
+ * The solve is the ik_controller op's damped least squares: at most max_iters iterations while the position residual of the last
+ * iterate exceeds `threshold`, on the URDF frame of link `link` (0 <= link < links of the body) in the coordinates of the base,
+ * whose pose is the state row's and stays fixed.
+ *   target_pos_dev [n_envs][3]            world position of the link frame
+ *   target_orn_dev [n_envs][4] or NULL     world orientation (xyzw, normalised here); NULL: position only (3 task rows)
+ *   q0_dev         [n_envs][nd] or NULL     seed (nd = the body's DoF); NULL: the state row's q
+ *   limits_dev     [n_envs][4][nd] or NULL  lower, upper, range, rest: adds the null-space term (SURVEY App. A.4); NULL: none
+ *   q_out_dev      [n_envs][nd]             the solution, the body's DoF in order
+ *   err_dev        [n_envs][2] or NULL      at q_out: distance of the link frame from the target (m), angle of the remaining
+ *                                           rotation (rad; 0 without target_orn)
+ * Writes nothing but the outputs and a scratch buffer the world allocates on the first call (calls on different streams must not
+ * overlap).  DG_E_ARG for no such body, a body without degrees of freedom, nd > DG_IK_MAX_ND, a link out of range,
+ * max_iters < 1, a negative or NaN threshold, or a NULL target_pos_dev / q_out_dev. */
+enum { DG_IK_MAX_ND = 64 };
+int dg_body_ik(DgWorld* w, int body, int link, const float* target_pos_dev, const float* target_orn_dev, const float* q0_dev,
+               const float* limits_dev, int max_iters, float threshold, float* q_out_dev, float* err_dev, void* stream);
+
 /* Host-buffer form of dg_step (the reference-facing call when the caller keeps numpy arrays): copies the actions
  * host->device, steps, copies obs / reward / terminal device->host and waits.  Any output pointer may be NULL. */
 int dg_step_host(DgWorld* w, const float* action_host, float* obs_host, float* reward_host, uint8_t* term_host, void* stream);
