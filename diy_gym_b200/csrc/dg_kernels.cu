@@ -383,65 +383,75 @@ __global__ void __launch_bounds__(256, 3) dg_render_kernel(const __grid_constant
   }
   __syncthreads();
   // ---- per-shape records (registers), keys, ranks, records to their sorted slot --------------------------------------------------
+  auto make_record = [&](int s, float* o) {
+    const int* vi = sc.vis_i + DG_VIS_I_W * s; const float* vf = sc.vis_f + DG_VIS_F_W * s;
+    if (vi[2]) { for (int i = 0; i < 12; i++) o[i] = sc.vis_wb[12 * s + i]; }
+    else {
+      float p[3], q[4], v[3], w[3], R[9], Rs[9], t[3];
+      frame_com_state(C, vi[0], p, q, v, w); q_to_mat(R, q); q_to_mat(Rs, vf + 3); m_mul(o, R, Rs);
+      m_vec(t, R, vf); v_add(o + 9, p, t);
+    }
+    for (int i = 0; i < 4; i++) o[12 + i] = vf[7 + i];
+    for (int i = 0; i < 3; i++) o[16 + i] = param[(size_t)e * sc.P + DG_PO(&sc, P_COLOR) + 3 * s + i];   // per-environment colour (visual_randomizer)
+    o[19] = int_as_float(vi[1]); o[20] = vf[15];
+    const float r = o[20];
+    float oc[3], ol[3]; v_sub(oc, camRp + 9, o + 9); mT_vec(ol, o, oc);
+    mT_mul(o + 21, o, camRp);                                   // camera-space direction -> shape-frame direction
+    o[30] = ol[0]; o[31] = ol[1]; o[32] = ol[2]; o[33] = v_dot(ol, ol) - r * r;
+    // oriented bounding box of the shape -> nearest eye-space depth and screen rectangle (whole screen if it reaches behind the eye)
+    const int type = vi[1]; const float* d = o + 12;
+    float hx = d[0], hy = d[1], hz = d[2];
+    if (type == SHAPE_SPHERE) { hy = d[0]; hz = d[0]; } else if (type == SHAPE_CAPSULE) { hy = d[0]; hz = d[1] + d[0]; } else if (type == SHAPE_CYLINDER) { hy = d[0]; hz = d[1]; }
+    // corners in camera space; the part of the box in front of the eye plane z = -zc is what can be seen: its screen rectangle
+    // comes from the corners in front and from the points where edges cross that plane
+    const float zc = fmaxf(0.5f * nearp, 1e-4f);
+    float ccx[8], ccy[8], ccd[8];
+    float zmin = 1e30f, x0 = 1e30f, x1 = -1e30f, y0 = 1e30f, y1 = -1e30f;
+    const float sx = 0.5f * width / (th * aspect), sy = 0.5f * height / th;
+    auto add_pt = [&](float cx, float cy, float dep) {
+      const float px = fminf(fmaxf(cx / dep * sx, -1e6f), 1e6f) + 0.5f * width - 0.5f, py = fminf(fmaxf(-cy / dep * sy, -1e6f), 1e6f) + 0.5f * height - 0.5f;
+      x0 = fminf(x0, px); x1 = fmaxf(x1, px); y0 = fminf(y0, py); y1 = fmaxf(y1, py);
+    };
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+      const float cl[3] = {(k & 1) ? hx : -hx, (k & 2) ? hy : -hy, (k & 4) ? hz : -hz};
+      float cw[3], rel[3], cc[3]; m_vec(cw, o, cl); v_add(cw, cw, o + 9); v_sub(rel, cw, camRp + 9); mT_vec(cc, camRp, rel);
+      ccx[k] = cc[0]; ccy[k] = cc[1]; ccd[k] = -cc[2];
+      zmin = fminf(zmin, ccd[k]);
+      if (ccd[k] > zc) add_pt(cc[0], cc[1], ccd[k]);
+    }
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+#pragma unroll
+      for (int bit = 1; bit < 8; bit <<= 1) {
+        if (k & bit) continue;
+        const int k2 = k | bit;
+        if ((ccd[k] > zc) == (ccd[k2] > zc)) continue;
+        const float t = (zc - ccd[k]) / (ccd[k2] - ccd[k]);
+        add_pt(ccx[k] + t * (ccx[k2] - ccx[k]), ccy[k] + t * (ccy[k2] - ccy[k]), zc);
+      }
+    }
+    if (x1 < x0) { x0 = y0 = 1e9f; x1 = y1 = -1e9f; }   // nothing of the box in front of the eye: never a candidate
+    zmin = fmaxf(zmin, 0.f);
+    o[VS_ZMIN] = zmin;
+    o[VS_RECT] = floorf(fmaxf(x0, -1e6f)) - 1.f; o[VS_RECT + 1] = ceilf(fminf(x1, 1e6f)) + 1.f;
+    o[VS_RECT + 2] = floorf(fmaxf(y0, -1e6f)) - 1.f; o[VS_RECT + 3] = ceilf(fminf(y1, 1e6f)) + 1.f;
+    o[VS_BODY] = (float)vi[3];
+  };
+  // a rank needs every key: with more shapes than threads the keys come first, in a pass of their own (each thread holds one
+  // record at a time, so those records are built twice), and the record pass takes its zmin from them
+  const bool one_pass = sc.nv <= (int)blockDim.x;
+  if (!one_pass) {
+    for (int s = threadIdx.x; s < sc.nv; s += blockDim.x) { float o[VS_W]; make_record(s, o); key[s] = o[VS_ZMIN]; }
+    __syncthreads();
+  }
   for (int s0 = 0; s0 < sc.nv; s0 += blockDim.x) {
     const int s = s0 + threadIdx.x; float o[VS_W];
     if (s < sc.nv) {
-      const int* vi = sc.vis_i + DG_VIS_I_W * s; const float* vf = sc.vis_f + DG_VIS_F_W * s;
-      if (vi[2]) { for (int i = 0; i < 12; i++) o[i] = sc.vis_wb[12 * s + i]; }
-      else {
-        float p[3], q[4], v[3], w[3], R[9], Rs[9], t[3];
-        frame_com_state(C, vi[0], p, q, v, w); q_to_mat(R, q); q_to_mat(Rs, vf + 3); m_mul(o, R, Rs);
-        m_vec(t, R, vf); v_add(o + 9, p, t);
-      }
-      for (int i = 0; i < 4; i++) o[12 + i] = vf[7 + i];
-      for (int i = 0; i < 3; i++) o[16 + i] = param[(size_t)e * sc.P + DG_PO(&sc, P_COLOR) + 3 * s + i];   // per-environment colour (visual_randomizer)
-      o[19] = int_as_float(vi[1]); o[20] = vf[15];
-      const float r = o[20];
-      float oc[3], ol[3]; v_sub(oc, camRp + 9, o + 9); mT_vec(ol, o, oc);
-      mT_mul(o + 21, o, camRp);                                   // camera-space direction -> shape-frame direction
-      o[30] = ol[0]; o[31] = ol[1]; o[32] = ol[2]; o[33] = v_dot(ol, ol) - r * r;
-      // oriented bounding box of the shape -> nearest eye-space depth and screen rectangle (whole screen if it reaches behind the eye)
-      const int type = vi[1]; const float* d = o + 12;
-      float hx = d[0], hy = d[1], hz = d[2];
-      if (type == SHAPE_SPHERE) { hy = d[0]; hz = d[0]; } else if (type == SHAPE_CAPSULE) { hy = d[0]; hz = d[1] + d[0]; } else if (type == SHAPE_CYLINDER) { hy = d[0]; hz = d[1]; }
-      // corners in camera space; the part of the box in front of the eye plane z = -zc is what can be seen: its screen rectangle
-      // comes from the corners in front and from the points where edges cross that plane
-      const float zc = fmaxf(0.5f * nearp, 1e-4f);
-      float ccx[8], ccy[8], ccd[8];
-      float zmin = 1e30f, x0 = 1e30f, x1 = -1e30f, y0 = 1e30f, y1 = -1e30f;
-      const float sx = 0.5f * width / (th * aspect), sy = 0.5f * height / th;
-      auto add_pt = [&](float cx, float cy, float dep) {
-        const float px = fminf(fmaxf(cx / dep * sx, -1e6f), 1e6f) + 0.5f * width - 0.5f, py = fminf(fmaxf(-cy / dep * sy, -1e6f), 1e6f) + 0.5f * height - 0.5f;
-        x0 = fminf(x0, px); x1 = fmaxf(x1, px); y0 = fminf(y0, py); y1 = fmaxf(y1, py);
-      };
-#pragma unroll
-      for (int k = 0; k < 8; k++) {
-        const float cl[3] = {(k & 1) ? hx : -hx, (k & 2) ? hy : -hy, (k & 4) ? hz : -hz};
-        float cw[3], rel[3], cc[3]; m_vec(cw, o, cl); v_add(cw, cw, o + 9); v_sub(rel, cw, camRp + 9); mT_vec(cc, camRp, rel);
-        ccx[k] = cc[0]; ccy[k] = cc[1]; ccd[k] = -cc[2];
-        zmin = fminf(zmin, ccd[k]);
-        if (ccd[k] > zc) add_pt(cc[0], cc[1], ccd[k]);
-      }
-#pragma unroll
-      for (int k = 0; k < 8; k++) {
-#pragma unroll
-        for (int bit = 1; bit < 8; bit <<= 1) {
-          if (k & bit) continue;
-          const int k2 = k | bit;
-          if ((ccd[k] > zc) == (ccd[k2] > zc)) continue;
-          const float t = (zc - ccd[k]) / (ccd[k2] - ccd[k]);
-          add_pt(ccx[k] + t * (ccx[k2] - ccx[k]), ccy[k] + t * (ccy[k2] - ccy[k]), zc);
-        }
-      }
-      if (x1 < x0) { x0 = y0 = 1e9f; x1 = y1 = -1e9f; }   // nothing of the box in front of the eye: never a candidate
-      zmin = fmaxf(zmin, 0.f);
-      o[VS_ZMIN] = zmin;
-      o[VS_RECT] = floorf(fmaxf(x0, -1e6f)) - 1.f; o[VS_RECT + 1] = ceilf(fminf(x1, 1e6f)) + 1.f;
-      o[VS_RECT + 2] = floorf(fmaxf(y0, -1e6f)) - 1.f; o[VS_RECT + 3] = ceilf(fminf(y1, 1e6f)) + 1.f;
-      o[VS_BODY] = (float)vi[3];
-      key[s] = zmin;
+      make_record(s, o);
+      if (one_pass) key[s] = o[VS_ZMIN]; else o[VS_ZMIN] = key[s];
     }
-    __syncthreads();
+    if (one_pass) __syncthreads();
     if (s < sc.nv) {
       int rank = 0; const float ks = key[s];
       for (int s2 = 0; s2 < sc.nv; s2++) { const float k2 = key[s2]; rank += (k2 < ks || (k2 == ks && s2 < s)) ? 1 : 0; }
@@ -701,12 +711,25 @@ struct DgWorld {
   unsigned long long graph_key[4] = {0, 0, 0, 0}; bool graph_valid = false;
   // ray_sensor ops (dg_ray_kernel, launched after the step / reset / observe launches when the scene has any)
   std::vector<int> ray_ops; size_t ray_smem = 0;
+  size_t render_static_smem = 0;       // largest static shared memory of the dg_render_kernel instantiations (scenes with cameras)
   // dg_body_ik: [n_envs][seed record + ik_stride] (dg_ik.cuh), allocated by the first call
   float* ik_rec = nullptr;
   int64_t launches = 0;
   std::string err;
 };
 static std::string g_create_err;
+
+// camera: the instantiation for a colour type, patch height (NH) and number of visual shapes (NCW = candidate words), and its
+// dynamic shared memory (records, keys, candidate bit set) - a block also has the kernel's static staging buffers
+using RenderFn = void (*)(DevScene, const float*, const float*, int, float*, float*, float*, int, int, int);
+static RenderFn render_kernel(bool u8, int nh, int nv) {
+  static const RenderFn table[2][2][3] = {
+      {{dg_render_kernel<1, 1, false>, dg_render_kernel<2, 1, false>, dg_render_kernel<4, 1, false>}, {dg_render_kernel<1, 2, false>, dg_render_kernel<2, 2, false>, dg_render_kernel<4, 2, false>}},
+      {{dg_render_kernel<1, 1, true>, dg_render_kernel<2, 1, true>, dg_render_kernel<4, 1, true>}, {dg_render_kernel<1, 2, true>, dg_render_kernel<2, 2, true>, dg_render_kernel<4, 2, true>}}};
+  const int ncw = (nv + 31) / 32;   // candidate words per patch the kernel keeps in registers: 1, 2 or 4 (then a per-shape tail)
+  return table[u8 ? 1 : 0][nh - 1][ncw <= 1 ? 0 : (ncw == 2 ? 1 : 2)];
+}
+static size_t render_dyn_smem(int nv) { return ((size_t)std::max(nv, 1) * VS_W + (size_t)((nv + 3) & ~3) + (size_t)(nv + 31) / 32 + 8) * sizeof(float); }
 
 // Every entry point runs on the world's own device, whatever the caller's current device is (two worlds on two GPUs in one
 // process, or a torch current device different from the world's), and leaves the caller's device as it found it.
@@ -874,6 +897,23 @@ int dg_world_create(const int32_t* ibuf, int n_ibuf, const double* fbuf, int n_f
       if (w->ray_smem > smem_cap || cudaFuncSetAttribute(dg_ray_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)w->ray_smem) != cudaSuccess) {
         g_create_err = "ray_sensor: the moving collision shapes do not fit in shared memory"; cudaGetLastError(); dg_world_destroy(w); return DG_E_NOMEM;
       }
+    }
+  }
+  if (w->hs.dev.ncam > 0) {
+    // camera: a render block holds a record of every visual shape (render_dyn_smem) beside the kernel's static buffers
+    const int nv = w->hs.dev.nv;
+    for (int u8 = 0; u8 < 2; u8++) for (int nh = 1; nh <= 2; nh++) {
+      cudaFuncAttributes fa;
+      if (cudaFuncGetAttributes(&fa, render_kernel(u8 != 0, nh, nv)) != cudaSuccess) {
+        g_create_err = "camera: cudaFuncGetAttributes of the render kernel failed"; cudaGetLastError(); dg_world_destroy(w); return DG_E_CUDA;
+      }
+      w->render_static_smem = std::max(w->render_static_smem, fa.sharedSizeBytes);
+    }
+    const size_t need = w->render_static_smem + render_dyn_smem(nv);
+    if (need > smem_cap) {
+      g_create_err = "camera: " + std::to_string(nv) + " visual shapes need " + std::to_string(need) + " B of shared memory per render block, the device allows " +
+                     std::to_string(smem_cap) + " B";
+      dg_world_destroy(w); return DG_E_NOMEM;
     }
   }
   *out = w;
@@ -1147,16 +1187,12 @@ static int render_any(DgWorld* w, int cam, void* rgb_dev, bool u8, float* depth_
   // those take 8 x 4 patches (measured: 50 x 50 is 14 % slower with the large ones, 200 x 200 12 % faster)
   const int nh = ((ci[1] + 7) / 8) * ((ci[2] + 7) / 8) >= 96 ? 2 : 1;
   int tiles_x = (ci[1] + 7) / 8, tiles_y = (ci[2] + 4 * nh - 1) / (4 * nh);
-  size_t smem = ((size_t)std::max(d.nv, 1) * VS_W + (size_t)((d.nv + 3) & ~3) + (size_t)(d.nv + 31) / 32 + 8) * sizeof(float);
-  const int ncw = (d.nv + 31) / 32;   // candidate words per patch the kernel keeps in registers: 1, 2 or 4 (then a per-shape tail)
+  const size_t smem = render_dyn_smem(d.nv);
   // (compiled for 3 resident blocks per SM, 80 registers; 4 blocks / 64 registers spills in the per-block set-up and measured
   // slower: 1.10 vs 1.03 ms per 4096 x 200 x 200 render)
-  using RenderFn = void (*)(DevScene, const float*, const float*, int, float*, float*, float*, int, int, int);
-  static const RenderFn table[2][2][3] = {
-      {{dg_render_kernel<1, 1, false>, dg_render_kernel<2, 1, false>, dg_render_kernel<4, 1, false>}, {dg_render_kernel<1, 2, false>, dg_render_kernel<2, 2, false>, dg_render_kernel<4, 2, false>}},
-      {{dg_render_kernel<1, 1, true>, dg_render_kernel<2, 1, true>, dg_render_kernel<4, 1, true>}, {dg_render_kernel<1, 2, true>, dg_render_kernel<2, 2, true>, dg_render_kernel<4, 2, true>}}};
-  RenderFn kern = table[u8 ? 1 : 0][nh - 1][ncw <= 1 ? 0 : (ncw == 2 ? 1 : 2)];
-  if (smem > 48 * 1024) { CK(w, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)w->smem_cap)); }
+  RenderFn kern = render_kernel(u8, nh, d.nv);
+  // above 48 KB of static + dynamic shared memory a block needs the opt-in (dg_world_create checked that it fits)
+  if (w->render_static_smem + smem > 48 * 1024) { CK(w, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); }
   // blocks per environment: one when the batch alone fills the GPU a few times over, else enough groups of tiles to do so
   int groups = std::max(1, std::min((tiles_x * tiles_y + 7) / 8, (8 * w->sm_count + w->n_envs - 1) / w->n_envs));
   w->launches++;

@@ -56,6 +56,8 @@ typedef struct DgBufferTable {
 /* Compile a scene for n_envs environments on CUDA device `device`.
  * (ibuf, fbuf) are the section buffers emitted by diy_gym_b200/compiler/scene.py (layout: csrc/scene_sections.h).
  * team = lanes per environment (1,2,4,8,16,32) or 0 for the built-in choice.
+ * DG_E_NOMEM when the scene does not fit the device's shared memory: the step workspace, the ray_sensor shapes, or a scene with
+ * a camera whose visual shapes' records exceed one render block (about 1350 visual shapes at 227 KB, DESIGN.md section 4.3).
  * Replaces: p.connect / p.resetSimulation / p.setPhysicsEngineParameter / p.setGravity / p.loadURDF ...
  *           (/root/reference/diy_gym/diy_gym.py:68-86, diy_gym/model.py:65-83) */
 int dg_world_create(const int32_t* ibuf, int n_ibuf, const double* fbuf, int n_fbuf, int n_envs, int device, int team,
@@ -101,7 +103,8 @@ int dg_render(DgWorld* w, int cam, float* rgb_dev, float* depth_dev, void* strea
  * the unique id (body index in load order) of the body visible in each pixel, -1 for the background; NULL = no mask. */
 int dg_render_seg(DgWorld* w, int cam, float* rgb_dev, float* depth_dev, float* seg_dev, void* stream);
 /* The same with the colour image as bytes: rgb_dev [n_envs][H][W][3] uint8 = round(255 c) - the renderer's own output format,
- * which the reference divides by 255 (sensors/camera.py:76-78); a quarter of the colour bytes to move.  seg_dev may be NULL. */
+ * which the reference divides by 255 (sensors/camera.py:76-78); a quarter of the colour bytes to move.  seg_dev may be NULL.
+ * All three render calls store whole 16-byte pieces: float buffers must be 16-byte aligned, colour bytes 8-byte aligned. */
 int dg_render_u8(DgWorld* w, int cam, uint8_t* rgb_dev, float* depth_dev, float* seg_dev, void* stream);
 
 /* Rigid-body dynamics of body `body` (load order) for every environment, from its state and parameter rows: one launch on `stream`.
