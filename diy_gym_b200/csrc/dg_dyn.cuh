@@ -12,7 +12,7 @@
 // Newton-Euler in world axes: tau = M qdd + C nu + G without forming M).  Masses and principal inertias come from the parameter
 // row (P_MASS, P_INERTIA: dynamics_randomizer is honoured); joint damping, motors, limits, contacts and welds are not included.
 //
-// The routines are DG_FN so that the test-only CPU build (tests/emul/dyn_emul.cpp) runs the same fp32 arithmetic as the kernel.
+// The routines are DG_FN so that the test-only CPU build (tests/emul/emul.cpp) runs the same fp32 arithmetic as the kernel.
 // One environment is evaluated in three phases: dyn_chain (one lane: the sequential pass over the links), dyn_links (lanes over
 // links: world inertias and the link wrenches), dyn_outputs (lanes over columns / matrix entries); a barrier between phases.
 #pragma once
@@ -35,6 +35,18 @@ struct DynArgs {
   const float *q, *qd, *qdd;        // [N][nd], [N][n], [N][n]; null: state row, state row, zero
   float *jac, *mass, *tau;          // [N][6][n] (linear rows first), [N][n][n], [N][n]; null: not computed
 };
+
+// The arguments of the queries of `body` (a valid index; host tables in sc).  n = 0 when the body has no degrees of freedom; the
+// caller checks n and link.  point null: the link's COM.
+inline DynArgs dyn_args(const DevScene& sc, int body, int link, const float* point, const float* q, const float* qd, const float* qdd,
+                        float* jac, float* mass, float* tau) {
+  const int* bi = sc.body_i + DG_BODY_I_W * body;
+  DynArgs a;
+  a.body = body; a.link = link; a.n = (bi[0] == 2 ? 6 : 0) + bi[4]; a.nl = bi[2] + 1;
+  for (int i = 0; i < 3; i++) a.point[i] = point ? point[i] : 0.f;
+  a.q = q; a.qd = qd; a.qdd = qdd; a.jac = jac; a.mass = mass; a.tau = tau;
+  return a;
+}
 
 // scratch of one environment: nl 64-bit column masks, then nl link records, n column records and the point (floats)
 DG_HD int dyn_scratch_floats(int nl, int n) { return (2 * nl + DL_W_ * nl + DC_W_ * n + 4 + 3) & ~3; }

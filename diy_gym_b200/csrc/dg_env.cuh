@@ -2172,4 +2172,12 @@ DG_FN void run_env_reset(const Env& C, int nt, DG_LANE_ARGS) {
 #endif
 }
 
+// The Env of a kernel that only reads state rows (camera, ray_sensor, IK query): the scene, the row st and the scene's link tables;
+// every other member null / zero.  (At the end of the file: the phase-timing keys of DG_PHASE are source lines.)
+DG_HD Env row_env(const DevScene& sc, float* st) {
+  Env C{};
+  C.sc = &sc; C.st = st; C.link_i = sc.link_i; C.link_f = sc.link_f; C.link_x = sc.link_x;
+  return C;
+}
+
 }  // namespace dg

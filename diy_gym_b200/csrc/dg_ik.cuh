@@ -9,8 +9,10 @@
 // entries of the queried body are written and read.  Afterwards ik_env evaluates the residual at the returned q with one more
 // pass of joint_xform over the chain.
 //
-// The routines are DG_FN so that the test-only CPU build (tests/emul/ik_emul.cpp) runs the same fp32 arithmetic as the kernel.
+// The routines are DG_FN so that the test-only CPU build (tests/emul/emul.cpp) runs the same fp32 arithmetic as the kernel.
 #pragma once
+#include <type_traits>
+
 #include "dg_env.cuh"
 
 namespace dg {
@@ -37,6 +39,29 @@ inline int ik_scene(DevScene& d, int iters, float threshold) {
   DG_SO(&d, S_Q) = 0; DG_SO(&d, S_BPOS) = d.nd; DG_SO(&d, S_BQUAT) = d.nd + 3 * d.nb;
   d.ik_iters = iters; d.ik_threshold = threshold;
   return (d.nd + 7 * d.nb + 3) & ~3;
+}
+
+// The arguments of the query of link `link` of `body` (validated by the caller; bi: the body's row of the body table, host memory),
+// and d, the copy of the scene the kernel gets, remapped by ik_scene.  The caller points rec at [N][rec_stride] floats.
+inline IkArgs ik_args(DevScene& d, const int* bi, int body, int link, const float* tpos, const float* torn, const float* q0,
+                      const float* lim, int iters, float threshold, float* q_out, float* err) {
+  IkArgs a;
+  a.body = body; a.link = bi[1] + link; a.use_orn = torn != nullptr;
+  a.s_q = DG_SO(&d, S_Q); a.s_bpos = DG_SO(&d, S_BPOS); a.s_bquat = DG_SO(&d, S_BQUAT);
+  a.seed_floats = ik_scene(d, iters, threshold);
+  a.rec_stride = a.seed_floats + d.ik_stride;
+  a.tpos = tpos; a.torn = torn; a.q0 = q0; a.lim = lim; a.q_out = q_out; a.err = err; a.rec = nullptr;
+  return a;
+}
+
+// The variant of the solve for a body of ndb DoF (the split of ik_solve_any): ik_solve_fast<MAXD, M> with its arrays in registers up
+// to 12 DoF (M = 6 with a target orientation, 3 without), the generic ik_solve (MAXD = M = 0) above.  Calls
+// f(std::integral_constant<int, MAXD>(), std::integral_constant<int, M>()).
+template <int N> using IkC = std::integral_constant<int, N>;
+template <class F> inline void ik_variant(int ndb, bool use_orn, F&& f) {
+  if (ndb <= 6) { if (use_orn) f(IkC<6>(), IkC<6>()); else f(IkC<6>(), IkC<3>()); }
+  else if (ndb <= 12) { if (use_orn) f(IkC<12>(), IkC<6>()); else f(IkC<12>(), IkC<3>()); }
+  else f(IkC<0>(), IkC<0>());
 }
 
 // Environment e: fill C.st (the seed record) from the arguments and the state row st, solve, write q_out and err.  MAXD = 0: the

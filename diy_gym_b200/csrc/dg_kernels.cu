@@ -34,15 +34,12 @@ struct LaunchArgs {
   int stages; float* carry; int* rs_lists; int* rs_count; unsigned* rs_used; int no_hot;   // rs_lists: [RS_NCLS][n_envs]
 };
 
-template <int T>
-__global__ void __launch_bounds__(256) dg_step_kernel(const __grid_constant__ DevScene sc, const LaunchArgs a) {
-  extern __shared__ __align__(16) float smem[];
-  // thread t = lane (t / E) of the block's environment (t % E): a warp holds one lane index of 32 environments
-  const int E = blockDim.x / T;
-  const int ei = threadIdx.x % E, ln = threadIdx.x / E;
-  Env C;
-  // the block's copy of the link tables sits behind the per-environment workspaces
-  int* s_link_i = reinterpret_cast<int*>(smem + (size_t)E * sc.w_total);
+// A block's shared-memory copy of the link tables (the step and IK kernels read them through shc()): link_i padded to a multiple of
+// four, then link_f and link_x.  link_table_floats: its size; stage_link_tables: the whole block copies the scene's tables to
+// `at`, waits for the copy and points C at it.
+__host__ __device__ inline int link_table_floats(int nl) { return ((DG_LINK_I_W * nl + 3) & ~3) + (DG_LINK_F_W + 16) * nl; }
+__device__ __forceinline__ void stage_link_tables(const DevScene& sc, float* at, Env& C) {
+  int* s_link_i = reinterpret_cast<int*>(at);
   float* s_link_f = reinterpret_cast<float*>(s_link_i + ((DG_LINK_I_W * sc.nl + 3) & ~3));
   float* s_link_x = s_link_f + DG_LINK_F_W * sc.nl;
   for (int i = threadIdx.x; i < DG_LINK_I_W * sc.nl; i += blockDim.x) s_link_i[i] = sc.link_i[i];
@@ -50,6 +47,16 @@ __global__ void __launch_bounds__(256) dg_step_kernel(const __grid_constant__ De
   for (int i = threadIdx.x; i < 16 * sc.nl; i += blockDim.x) s_link_x[i] = sc.link_x[i];
   __syncthreads();
   C.link_i = s_link_i; C.link_f = s_link_f; C.link_x = s_link_x;
+}
+
+template <int T>
+__global__ void __launch_bounds__(256) dg_step_kernel(const __grid_constant__ DevScene sc, const LaunchArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  // thread t = lane (t / E) of the block's environment (t % E): a warp holds one lane index of 32 environments
+  const int E = blockDim.x / T;
+  const int ei = threadIdx.x % E, ln = threadIdx.x / E;
+  Env C;
+  stage_link_tables(sc, smem + (size_t)E * sc.w_total, C);   // behind the per-environment workspaces
   C.sc = &sc; C.ws = smem + (size_t)ei * sc.w_total; C.seed = a.seed;
   C.opmask[0] = a.opmask[0]; C.opmask[1] = a.opmask[1]; C.dbg = a.dbg; C.dropped = a.dropped;
   C.split = a.stages != ST_ALL ? 1 : 0; C.rs_lists = a.rs_lists; C.rs_stride = a.n_envs; C.rs_count = a.rs_count; C.rs_used = a.rs_used; C.no_hot = a.no_hot;
@@ -372,8 +379,7 @@ __global__ void __launch_bounds__(256, 3) dg_render_kernel(const __grid_constant
   const int* ci = sc.cam_i + DG_CAM_I_W * cam; const float* cf = sc.cam_f + DG_CAM_F_W * cam;
   const int width = ci[1], height = ci[2];
   float* key = vs + VS_W * sc.nv;
-  Env C; C.sc = &sc; C.st = const_cast<float*>(state) + (size_t)e * sc.S; C.ws = nullptr; C.wg = nullptr; C.pr = nullptr; C.dbg = nullptr; C.dropped = nullptr; C.rs_used = nullptr; C.no_hot = 0;
-  C.link_i = sc.link_i; C.link_f = sc.link_f; C.link_x = sc.link_x;
+  const Env C = row_env(sc, const_cast<float*>(state) + (size_t)e * sc.S);
   const float fov = cf[7], nearp = cf[8], farp = cf[9];
   const float th = tanf(fov * kPi / 360.0f), aspect = (float)width / (float)height;
   if (threadIdx.x == 0) {
@@ -607,9 +613,8 @@ __global__ void __launch_bounds__(32 * kRayWarps) dg_ray_kernel(const __grid_con
   const int e = blockIdx.x * kRayWarps + warp;
   if (e >= n_envs || (mask != nullptr && mask[e] == 0)) return;   // (whole warps: no barrier below spans more than one)
   float* mov = ray_mov + (size_t)warp * 12 * sc.nshw;
-  Env C; C.sc = &sc; C.st = const_cast<float*>(state) + (size_t)e * sc.S; C.obs = obs + (size_t)e * sc.n_obs;
-  C.ws = nullptr; C.wg = nullptr; C.pr = nullptr; C.dbg = nullptr; C.dropped = nullptr; C.rs_used = nullptr; C.no_hot = 0;
-  C.link_i = sc.link_i; C.link_f = sc.link_f; C.link_x = sc.link_x;
+  Env C = row_env(sc, const_cast<float*>(state) + (size_t)e * sc.S);
+  C.obs = obs + (size_t)e * sc.n_obs;
   ray_stage_shapes(C, mov, lane, 32);
   __syncwarp();
   ray_env(C, mov, lane, 32);
@@ -645,18 +650,11 @@ __global__ void __launch_bounds__(32 * kDynWarps) dg_dyn_kernel(const __grid_con
 constexpr int kIkThreads = 64;
 template <int MAXD, int M>
 __global__ void __launch_bounds__(kIkThreads) dg_ik_kernel(const __grid_constant__ DevScene sc, const IkArgs a, const float* state, int n_envs) {
-  extern __shared__ __align__(16) float ik_smem[];
-  int* s_link_i = reinterpret_cast<int*>(ik_smem);
-  float* s_link_f = reinterpret_cast<float*>(s_link_i + ((DG_LINK_I_W * sc.nl + 3) & ~3));
-  float* s_link_x = s_link_f + DG_LINK_F_W * sc.nl;
-  for (int i = threadIdx.x; i < DG_LINK_I_W * sc.nl; i += blockDim.x) s_link_i[i] = sc.link_i[i];
-  for (int i = threadIdx.x; i < DG_LINK_F_W * sc.nl; i += blockDim.x) s_link_f[i] = sc.link_f[i];
-  for (int i = threadIdx.x; i < 16 * sc.nl; i += blockDim.x) s_link_x[i] = sc.link_x[i];
-  __syncthreads();
+  extern __shared__ __align__(16) float ik_smem[];   // [link_table_floats(nl)]
+  Env C = row_env(sc, nullptr);
+  stage_link_tables(sc, ik_smem, C);
   const int e = blockIdx.x * kIkThreads + threadIdx.x;
   if (e >= n_envs) return;
-  Env C;
-  C.sc = &sc; C.link_i = s_link_i; C.link_f = s_link_f; C.link_x = s_link_x;
   C.st = a.rec + (size_t)e * a.rec_stride;
   float scr[IkFastScratch<MAXD>::floats];
   ik_env<MAXD, M>(C, a, state + (size_t)e * sc.S, e, scr);
@@ -843,7 +841,7 @@ int dg_world_create(const int32_t* ibuf, int n_ibuf, const double* fbuf, int n_f
   {
     size_t per_team = (size_t)w->hs.dev.w_total * sizeof(float);
     const int nl_ = w->hs.dev.nl;
-    size_t tables = (size_t)(((DG_LINK_I_W * nl_ + 3) & ~3) + (DG_LINK_F_W + 16) * nl_ + 4) * sizeof(float);   // block-shared link tables
+    size_t tables = (size_t)(link_table_floats(nl_) + 4) * sizeof(float);   // block-shared link tables
     int teams = block / team;
     while (teams > 1 && per_team * teams + tables > smem_cap) teams--;
     if (per_team * teams + tables > smem_cap) { g_create_err = "scene workspace (" + std::to_string(per_team) + " B per environment) exceeds shared memory"; delete w; return DG_E_NOMEM; }
@@ -1124,13 +1122,10 @@ int dg_body_dynamics(DgWorld* w, int body, int link, const float point[3], const
   const DevScene& hd = w->hs.dev;   // (host pointers)
   if (body < 0 || body >= hd.nb) { w->err = "dg_body_dynamics: no such body"; return DG_E_ARG; }
   const int* bi = hd.body_i + DG_BODY_I_W * body;
-  DynArgs a;
-  a.body = body; a.link = link; a.n = (bi[0] == 2 ? 6 : 0) + bi[4]; a.nl = bi[2] + 1;
+  const DynArgs a = dyn_args(hd, body, link, point, q_dev, qd_dev, qdd_dev, jac_dev, mass_dev, tau_dev);
   if (bi[0] == 0 || a.n == 0) { w->err = "dg_body_dynamics: the body has no degrees of freedom"; return DG_E_ARG; }
   if (a.n > DG_DYN_MAXN) { w->err = "dg_body_dynamics: the body has " + std::to_string(a.n) + " generalized coordinates, more than " + std::to_string((int)DG_DYN_MAXN); return DG_E_ARG; }
   if (link < -1 || link >= bi[2]) { w->err = "dg_body_dynamics: no such link"; return DG_E_ARG; }
-  for (int i = 0; i < 3; i++) a.point[i] = point ? point[i] : 0.f;
-  a.q = q_dev; a.qd = qd_dev; a.qdd = qdd_dev; a.jac = jac_dev; a.mass = mass_dev; a.tau = tau_dev;
   if (!jac_dev && !mass_dev && !tau_dev) return DG_OK;
   DeviceGuard guard(w->device);
   const size_t smem = (size_t)kDynWarps * dyn_scratch_floats(a.nl, a.n) * sizeof(float);
@@ -1156,21 +1151,15 @@ int dg_body_ik(DgWorld* w, int body, int link, const float* target_pos_dev, cons
   if (!(threshold >= 0.f)) { w->err = "dg_body_ik: threshold must be a number >= 0"; return DG_E_ARG; }
   if (!target_pos_dev || !q_out_dev) { w->err = "dg_body_ik: target_pos and q_out are required"; return DG_E_ARG; }
   DevScene d = w->dev;   // (device pointers)
-  IkArgs a;
-  a.body = body; a.link = bi[1] + link; a.use_orn = target_orn_dev != nullptr;
-  a.s_q = DG_SO(&d, S_Q); a.s_bpos = DG_SO(&d, S_BPOS); a.s_bquat = DG_SO(&d, S_BQUAT);
-  a.seed_floats = ik_scene(d, max_iters, threshold);
-  a.rec_stride = a.seed_floats + d.ik_stride;
-  a.tpos = target_pos_dev; a.torn = target_orn_dev; a.q0 = q0_dev; a.lim = limits_dev; a.q_out = q_out_dev; a.err = err_dev;
+  IkArgs a = ik_args(d, bi, body, link, target_pos_dev, target_orn_dev, q0_dev, limits_dev, max_iters, threshold, q_out_dev, err_dev);
   DeviceGuard guard(w->device);
   if (!w->ik_rec) CK(w, cudaMalloc(&w->ik_rec, (size_t)w->n_envs * a.rec_stride * sizeof(float)));
   a.rec = w->ik_rec;
-  const size_t smem = (size_t)(((DG_LINK_I_W * d.nl + 3) & ~3) + (DG_LINK_F_W + 16) * d.nl) * sizeof(float);
-  const cudaStream_t s = (cudaStream_t)stream;
-  // the split of ik_solve_any: register-resident solves up to 12 DoF, the generic one above
-  auto launch = ndb <= 6 ? (a.use_orn ? ik_launch<6, 6> : ik_launch<6, 3>) : ndb <= 12 ? (a.use_orn ? ik_launch<12, 6> : ik_launch<12, 3>) : ik_launch<0, 0>;
+  const size_t smem = (size_t)link_table_floats(d.nl) * sizeof(float);
+  cudaError_t e = cudaSuccess;
+  ik_variant(ndb, a.use_orn, [&](auto maxd, auto m) { e = ik_launch<decltype(maxd)::value, decltype(m)::value>(d, a, w->buf.state, w->n_envs, smem, (cudaStream_t)stream); });
   w->launches++;
-  CK(w, launch(d, a, w->buf.state, w->n_envs, smem, s));
+  CK(w, e);
   return DG_OK;
 }
 int dg_reset(DgWorld* w, const uint8_t* mask_dev, void* stream) { return run(w, 1, mask_dev, stream); }

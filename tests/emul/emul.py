@@ -1,5 +1,5 @@
-"""ctypes wrapper of the CPU emulation of the device step code (tests/emul/emul.cpp).  TEST INFRASTRUCTURE:
-lets the GPU-less container check the kernel logic (fp32, team phases) against the fp64 oracle."""
+"""ctypes wrapper of the CPU emulation of the device code (tests/emul/emul.cpp).  TEST INFRASTRUCTURE: lets the GPU-less
+container check the kernel logic (fp32, team phases, ray / dynamics / IK queries) against the fp64 oracle and references."""
 import ctypes
 import os
 import subprocess
@@ -12,10 +12,15 @@ _LIB = None
 
 
 def build(force=False):
+    """The emulation library, rebuilt when emul.cpp or any file of the device code is newer.  Written under a name of its own
+    and renamed into place, so that test processes running side by side never load a half-written library."""
     so = os.path.join(_HERE, 'libdgemul.so')
-    srcs = [os.path.join(_HERE, 'emul.cpp')] + [os.path.join(_CSRC, f) for f in ('dg_env.cuh', 'dg_math.cuh', 'dg_scene.h', 'scene_sections.h')]
+    src = os.path.join(_HERE, 'emul.cpp')
+    srcs = [src] + [os.path.join(_CSRC, f) for f in os.listdir(_CSRC)]
     if force or not os.path.isfile(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        subprocess.check_call(['g++', '-O2', '-fPIC', '-shared', '-std=c++17', '-Wno-unknown-pragmas', '-o', so, srcs[0]])
+        tmp = '%s.%d.tmp' % (so, os.getpid())
+        subprocess.check_call(['g++', '-O2', '-fPIC', '-shared', '-std=c++17', '-Wno-unknown-pragmas', '-o', tmp, src])
+        os.replace(tmp, so)
     return so
 
 
@@ -44,12 +49,19 @@ def lib():
         L.dge_observe.argtypes = [vp, fp, fp, u8]
         L.dge_contacts_dropped.restype = ctypes.c_uint
         L.dge_contacts_dropped.argtypes = [vp]
+        L.dge_rays.argtypes = [vp, fp, fp, ctypes.c_int, u8]
+        L.dge_dynamics.argtypes = [vp, ctypes.c_int, ctypes.c_int, fp, fp, fp, fp, fp, fp, fp, fp, fp, ctypes.c_int]
+        L.dge_ik.argtypes = [vp, ctypes.c_int, ctypes.c_int, fp, fp, fp, fp, ctypes.c_int, ctypes.c_float, fp, fp, fp, ctypes.c_int]
         _LIB = L
     return _LIB
 
 
 def _fp(a):
-    return a.ctypes.data_as(ctypes.POINTER(ctypes.c_float))
+    return None if a is None else a.ctypes.data_as(ctypes.POINTER(ctypes.c_float))
+
+
+def _f32(a):
+    return None if a is None else np.ascontiguousarray(a, np.float32)
 
 
 class EmulWorld:
@@ -115,3 +127,39 @@ class EmulWorld:
 
     def physics(self, nsub=None):
         lib().dge_physics(self._w, self.h['substeps'] if nsub is None else nsub)
+
+    # The kernels that read state rows, on explicit rows (numpy, any float dtype) rather than the world's own.
+    def rays(self, state, obs=None, mask=None):
+        """The ray_sensor ops (dg_ray_kernel) from state rows [n, S] into the ray slices of observation rows [n, n_obs]: in place
+        when obs (float32, C-contiguous) is given, else into fresh rows that hold only the rays.  mask: only those environments."""
+        h = self.h
+        state = np.ascontiguousarray(np.atleast_2d(state), np.float32)
+        if obs is None:
+            obs = np.zeros((len(state), max(h['n_obs'], 1)), np.float32)
+        assert obs.dtype == np.float32 and obs.flags.c_contiguous and state.shape[1] == h['S']
+        assert obs.shape[1] >= h['n_obs'] and (obs.shape[1] == max(h['n_obs'], 1) or len(obs) == 1)   # (the C side's row stride: n_obs)
+        m = None if mask is None else np.ascontiguousarray(mask, np.uint8)
+        lib().dge_rays(self._w, _fp(state), _fp(obs), len(state), None if m is None else m.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)))
+        return obs[:, :h['n_obs']]
+
+    def dynamics(self, state, param, body, link=-1, point=(0., 0., 0.), q=None, qd=None, qdd=None, jac=True, mass=True, tau=True):
+        """dg_dyn_kernel: (jac [N,6,n], mass [N,n,n], tau [N,n]) as numpy float32 (None where not asked for)."""
+        b = self.scene.bodies[body]
+        n = b.n_dofs + (6 if b.kind == 2 else 0)
+        state, param, point, q, qd, qdd = _f32(state), _f32(param), _f32(point), _f32(q), _f32(qd), _f32(qdd)
+        N = len(state)
+        outs = [np.zeros((N, 6, n), np.float32) if jac else None, np.zeros((N, n, n), np.float32) if mass else None,
+                np.zeros((N, n), np.float32) if tau else None]
+        lib().dge_dynamics(self._w, int(body), int(link), _fp(point), _fp(q), _fp(qd), _fp(qdd), *[_fp(o) for o in outs],
+                           _fp(state), _fp(param), N)
+        return tuple(outs)
+
+    def ik(self, state, body, link, tpos, torn=None, q=None, limits=None, iters=20, threshold=1e-4):
+        """dg_ik_kernel: (q [N, n_dof], err [N, 2]) as numpy float32; tpos [N, 3], torn [N, 4], q [N, n_dof], limits [N, 4, n_dof] or
+        None."""
+        nd, N = self.scene.bodies[body].n_dofs, len(state)
+        state, tpos, torn, q, limits = _f32(state), _f32(tpos), _f32(torn), _f32(q), _f32(limits)
+        q_out, err = np.zeros((N, nd), np.float32), np.zeros((N, 2), np.float32)
+        lib().dge_ik(self._w, int(body), int(link), _fp(tpos), _fp(torn), _fp(q), _fp(limits), int(iters), float(threshold), _fp(q_out),
+                     _fp(err), _fp(state), N)
+        return q_out, err

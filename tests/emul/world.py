@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE: a CPU stand-in with the interface of diy_gym_b200.backend.World, backed by the g++ build
-of the device step code (tests/emul/emul.cpp) and, for camera images, by the oracle's ray caster.  It lets the
+of the device code (tests/emul/emul.cpp) and, for camera images, by the oracle's ray caster.  It lets the
 GPU-less container exercise the whole host layer (DIYGym, Model, add-ons); the product never uses it."""
 import ctypes
 
@@ -8,6 +8,10 @@ import torch
 
 from oracle.oracle import OracleWorld
 from .emul import EmulWorld, _fp, lib
+
+
+def _np(t):
+    return None if t is None else t.detach().cpu().numpy()
 
 
 class EmulTorchWorld:
@@ -35,9 +39,11 @@ class EmulTorchWorld:
     def _ptrs(self):
         return _fp(self._o), _fp(self._r), self._t.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
+    # step / reset / observe cast the ray_sensor rays afterwards, as the backend's launches do (a reset: the masked environments only)
     def step(self):
         self.launches += 1
         lib().dge_step(self.e._w, _fp(self._a), *self._ptrs())
+        self.e.rays(self.e.state, self._o)
 
     def set_seed(self, seed, env_id_offset=0):
         lib().dge_set_seed(self.e._w, int(seed) & 0xffffffff, int(env_id_offset))
@@ -45,17 +51,24 @@ class EmulTorchWorld:
     def observe(self):
         self.launches += 1
         lib().dge_observe(self.e._w, *self._ptrs())
+        self.e.rays(self.e.state, self._o)
 
     def contacts_dropped(self):
         return self.e.contacts_dropped()
 
     def reset(self, mask=None):
         self.launches += 1
-        m = None
-        if mask is not None:
-            self._m = np.ascontiguousarray(mask.to(torch.uint8).cpu().numpy())
-            m = self._m.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
-        lib().dge_reset(self.e._w, m, *self._ptrs())
+        m = None if mask is None else np.ascontiguousarray(mask.to(torch.uint8).cpu().numpy())
+        lib().dge_reset(self.e._w, None if m is None else m.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), *self._ptrs())
+        self.e.rays(self.e.state, self._o, m)
+
+    def body_dynamics(self, body, link=-1, point=(0., 0., 0.), q=None, qd=None, qdd=None, jac=False, mass=False, tau=False):
+        out = self.e.dynamics(self.e.state, self.e.param, body, link, point, _np(q), _np(qd), _np(qdd), jac, mass, tau)
+        return tuple(None if o is None else torch.from_numpy(o) for o in out)
+
+    def body_ik(self, body, link, target_pos, target_orn=None, q=None, limits=None, max_iters=20, threshold=1e-4, err=False):
+        q_out, e = self.e.ik(self.e.state, body, link, _np(target_pos), _np(target_orn), _np(q), _np(limits), max_iters, threshold)
+        return torch.from_numpy(q_out), torch.from_numpy(e) if err else None
 
     def render(self, cam=0, seg=False, u8=False):
         if self._oracle is None:

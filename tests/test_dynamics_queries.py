@@ -2,7 +2,7 @@
 calculateMassMatrix / calculateInverseDynamics, csrc/dg_dyn.cuh + dg_dyn_kernel), apply_joint_torque and disable_motors.
 
 CPU: the fp64 reference (tests/dynamics_reference.py) is pinned by known answers and by the oracle's forward dynamics; the g++
-build of dg_dyn.cuh (tests/emul/dyn_emul.py) is checked against it on the example scenes; the host layer runs on the emulated
+build of dg_dyn.cuh (tests/emul) is checked against it on the example scenes; the host layer runs on the emulated
 world, including the reference's admittance controller written as a user add-on on these queries.  GPU: the same checks on the
 kernel, plus J nu against the step kernel's link-velocity cache, side effects and streams."""
 import os
@@ -42,7 +42,7 @@ def _env(folder, name, n, factory=None, path=None):
 
 
 def _emul_env(folder, name, n=4, path=None):
-    from tests.emul.dyn_emul import factory
+    from tests.emul.world import factory
     return _env(folder, name, n, factory(4), path)
 
 
@@ -394,7 +394,7 @@ def _admittance_parity(tmp_path, factory, n):
 
 
 def test_admittance_controller_as_user_addon(tmp_path):
-    from tests.emul.dyn_emul import factory
+    from tests.emul.world import factory
     _admittance_parity(tmp_path, factory(4), 4)
 
 

@@ -1,7 +1,7 @@
 """Batched inverse kinematics of a Model (pybullet's calculateInverseKinematics: csrc/dg_ik.cuh + dg_ik_kernel over the step
 kernel's ik_solve*) and position-motor targets (setJointMotorControlArray(POSITION_CONTROL)).
 
-CPU: the fp64 reference (tests/ik_reference.py) is pinned to the oracle's IK; the g++ build of dg_ik.cuh (tests/emul/ik_emul.py)
+CPU: the fp64 reference (tests/ik_reference.py) is pinned to the oracle's IK; the g++ build of dg_ik.cuh (tests/emul)
 is checked against it on every template path; known answers; the host layer and its errors on the emulated world; the
 reference's ik_controller written as a user add-on on these calls; set_position_targets against joint_controller.  GPU: the same
 checks on the kernel, plus side effects and streams."""
@@ -41,7 +41,7 @@ def _env(folder, name, n, factory=None, path=None):
 
 
 def _emul_factory(team=4):
-    from tests.emul.ik_emul import factory
+    from tests.emul.world import factory
     return factory(team)
 
 

@@ -1,5 +1,5 @@
 """ray_sensor add-on: host layer (pattern, spaces, validation), known answers of the fp64 reference (tests/ray_reference.py), the
-fp32 device routines (g++ build, tests/emul/ray_emul.py) against it, and on the GPU the CUDA kernel through the C ABI against it and
+fp32 device routines (g++ build, tests/emul) against it, and on the GPU the CUDA kernel through the C ABI against it and
 against itself across schedules.  The oracle world (oracle/) is used for what it already offers: forward kinematics into the link
 cache of a state row, and the step physics of the emulated legs."""
 import os
@@ -18,7 +18,6 @@ from diy_gym_b200.addons.builtin import RaySensor
 from oracle.oracle import OracleWorld
 from tests import ray_reference
 from tests.emul.emul import EmulWorld
-from tests.emul.ray_emul import RayCaster
 from tools.ray_probe import maze_with_lidar, ray_ops
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -111,7 +110,7 @@ def test_environment_level_sensor_rejects_a_frame():
 
 
 def test_host_layer_on_emulated_world_nested_flattened_and_terminal_observation():
-    from tests.emul.ray_emul import factory
+    from tests.emul.world import factory
     env = DIYGym(Configuration.from_dict('ray_sensor', example_config()), num_envs=2, world_factory=factory())
     obs = env.reset()
     d, h = obs['r2d2']['lidar']['distance'], obs['r2d2']['lidar']['hit_object']
@@ -142,6 +141,32 @@ def test_host_layer_on_emulated_world_nested_flattened_and_terminal_observation(
     assert torch.equal(obs_a['r2d2']['lidar']['distance'], enva.world.obs[:, :64])   # the rays of the fresh episode
 
 
+def test_emulated_world_casts_rays_after_reset_step_and_observe():
+    """The stand-in world's launches cast the rays as the backend's do: its observation rows hold what EmulWorld.rays casts from
+    the same state rows, after a reset (the masked environments only), a step and an observe."""
+    from tests.emul.world import factory
+    env = DIYGym(Configuration.from_dict('ray_sensor', example_config()), num_envs=3, world_factory=factory())
+    w = env.world
+    cols = np.concatenate([np.arange(off, off + (2 * R if hit else R)) for off, R, hit in ray_ops(env.scene)])
+
+    def check():
+        obs = w.obs.numpy()
+        assert np.array_equal(obs[:, cols], w.e.rays(w.e.state)[:, cols])
+        assert (obs[:, cols[:64]] > 0).all()   # distances (the rows start out zero)
+    w.reset()
+    check()
+    w.obs.fill_(-7.0)
+    w.reset(torch.tensor([0, 1, 0]))
+    assert (w.obs.numpy()[[0, 2]][:, cols] == -7.0).all()
+    assert np.array_equal(w.obs.numpy()[1, cols], w.e.rays(w.e.state[1])[0, cols])
+    w.action.uniform_(-0.5, 0.5)
+    w.step()
+    check()
+    w.obs.fill_(-7.0)
+    w.observe()
+    check()
+
+
 # ---------------------------------------------------------------- known answers of the fp64 reference --------------
 URDF = '''<robot name="k"><link name="base"><inertial><mass value="1"/><inertia ixx="1" ixy="0" ixz="0" iyy="1" iyz="0" izz="1"/></inertial>
 <collision><origin xyz="0 0 0" rpy="0 0 0"/><geometry>%s</geometry></collision></link></robot>'''
@@ -169,7 +194,7 @@ def _cast(scene, origin, quat=(0, 0, 0, 1)):
     o.s('S_BQUAT', 4)[:] = quat
     o.refresh()
     obs = ray_reference.cast(scene, o.state)
-    em = RayCaster(scene).rays(o.state)[0]
+    em = EmulWorld(scene).rays(o.state)[0]
     R = len(obs) // 2
     np.testing.assert_allclose(em[:R], obs[:R], atol=2e-5, rtol=1e-5)
     np.testing.assert_array_equal(em[R:], obs[R:])
@@ -306,7 +331,7 @@ def test_hit_ids_and_sensor_on_head_swivel_turns_with_q(tmp_path):
         org = pos + R @ [0.3, 0, 0.45]
         d, hb = ray_reference.cast(sc, o.state)
         out[q] = (d, hb, org)
-        em = RayCaster(sc).rays(o.state)[0]
+        em = EmulWorld(sc).rays(o.state)[0]
         assert abs(em[0] - d) < 2e-5 and em[1] == hb
     d, hb, org = out[0.0]
     assert hb == 1 and abs(d - (3.9 - org[0])) < 1e-9
@@ -345,13 +370,13 @@ def parity(scene, states, obs):
 def _emul_run(cfg, n, steps, seed=5):
     env = DIYGym(cfg, num_envs=1, compile_only=True)
     sc = env.scene
-    e, rays = EmulWorld(sc, n, team=4, seed=seed), RayCaster(sc)
+    e = EmulWorld(sc, n, team=4, seed=seed)
     e.reset()
-    yield sc, e.state.copy(), rays.rays(e.state)
+    yield sc, e.state.copy(), e.rays(e.state)
     rng = np.random.default_rng(seed)
     for _ in range(steps):
         e.step(rng.uniform(-0.5, 0.5, size=(n, sc.hdr['n_act'])).astype(np.float32))
-    yield sc, e.state.copy(), rays.rays(e.state)
+    yield sc, e.state.copy(), e.rays(e.state)
 
 
 @pytest.mark.parametrize('which', ['example', 'maze_lidar'])
